@@ -2,6 +2,7 @@
 """bench.py -- megapixels/sec of the stage 01-03 hot path (resize + colour layers + edges) on B200.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload config5|config2|config3|config4]
+                    [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one image per GPU: 01 resize_if_needed (a no-op for the
 named config, exactly as in the reference: max_dimension = image size), 02 nearest-centre assignment
@@ -212,9 +213,29 @@ STAGES = {"color": ("build_cells", "build_rgbcells", "build_tables", "assign_bit
           "edge": ("edge_runs", "edges3_bits", "hysteresis_bits", "morph", "blur", "canny_nms", "hyst_pass", "hyst_final")}
 
 
-def measure_fused(torch, eng, wl, img, centers, lut, steps, warmup, flush, barrier, cache_tables):
+DUMP_BYTES = 64 * 10**6
+
+
+def output_sample(torch, outs, seed=0):
+    """--dump-outputs: the u8 planes a caller of the timed call receives, as float32 arrays.  An output that fits its share of
+    DUMP_BYTES is kept whole; a larger one by its values at a fixed, seeded set of flat positions (the same for the same
+    workload on every run), beside `<name>_nonzero`, the nonzero count of every plane of the whole output."""
+    per = (DUMP_BYTES - 10**6) // 4 // len(outs)
+    res = {}
+    for name, t in outs.items():
+        n = t.numel()
+        if n <= per:
+            res[name] = t.float().cpu().numpy()
+        else:
+            pos = np.unique(np.random.default_rng(seed).integers(0, n, per))
+            res[name] = t.reshape(-1)[torch.from_numpy(pos).to(t.device)].float().cpu().numpy()
+        res[name + "_nonzero"] = t.reshape(t.shape[:-2] + (-1,)).count_nonzero(-1).double().cpu().numpy()
+    return res
+
+
+def measure_fused(torch, eng, wl, img, centers, lut, steps, warmup, flush, barrier, cache_tables, dump=False):
     """Device-resident fused call on one image (or one frame batch): CUDA events per step, L2 flushed (untimed) between steps,
-    then a second pass of the same steps with per-kernel events."""
+    then a second pass of the same steps with per-kernel events.  dump: also return device copies of the last timed step's outputs."""
     import omni_b200
     h, w, K = wl["h"], wl["w"], wl["K"]
     B = int(wl.get("batch", 1))
@@ -246,6 +267,7 @@ def measure_fused(torch, eng, wl, img, centers, lut, steps, warmup, flush, barri
     barrier()
     wall = time.perf_counter() - t0
     launches = eng.launch_count() - n0
+    last = {"masks": d_masks.clone(), "edges": d_edges.clone()} if dump else None
     eng.profile(True)
     pev = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(steps)]
     for a, b in pev:
@@ -260,7 +282,7 @@ def measure_fused(torch, eng, wl, img, centers, lut, steps, warmup, flush, barri
     step_ms = [a.elapsed_time(b) for a, b in ev]
     return {"step_ms": step_ms, "total_ms": sum(step_ms), "launches": launches, "prof": prof,
             "prof_step_ms": sum(a.elapsed_time(b) for a, b in pev) / steps, "wall": wall, "passes": eng.last_hysteresis_passes(),
-            "d_edges": d_edges, "ec": ec}
+            "d_edges": d_edges, "ec": ec, "last": last}
 
 
 def roofline_record(prof, prof_step_ms, ms_per_step, steps, N, K, workload, peak, peak_src):
@@ -487,8 +509,13 @@ def run_ours(args, wl):
     sampler = ClockSampler(physical_gpu_index(local))
     sampler.start()
     time.sleep(0.05)
-    m = measure_fused(torch, eng, wl, frames, centers, lut, args.steps, args.warmup, flush, barrier, cache_tables=(B > 1))
+    m = measure_fused(torch, eng, wl, frames, centers, lut, args.steps, args.warmup, flush, barrier, cache_tables=(B > 1),
+                      dump=bool(args.dump_outputs) and rank == 0)
     clocks = sampler.result()
+    if m["last"] is not None:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in output_sample(torch, m.pop("last")).items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
     t = torch.tensor([m["total_ms"]], dtype=torch.float64, device="cuda")
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -694,7 +721,12 @@ def main():
     ap.add_argument("--workload", choices=sorted(WORKLOADS), default="config5")
     ap.add_argument("--frames", type=int, default=512, help="frames of the configs[3] batch record")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the masks and edges of the last timed step (rank 0) to DIR/<name>.npy as float32, "
+                         "a fixed seeded sample of them when they exceed 64 MB, to compare two builds output for output")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     wl = WORKLOADS[args.workload]
     if args.gpus > 1 and "WORLD_SIZE" not in os.environ:
         # launched directly with --gpus N: re-launch one rank per GPU the way the driver does

@@ -1,7 +1,8 @@
-"""oracle/refport.py must compute what the reference's own functions compute.  Needs
-/root/reference (build container only) -- elsewhere these are skipped and the frozen golden
-fixtures (test_oracle_golden.py) carry the pin."""
+"""oracle/refport.py must compute what the reference's own functions compute: checked against outputs of the unmodified
+reference frozen under tests/golden/ (tools/make_golden.py, tools/make_golden_process_colors.py).  The stage-04 swap-point
+test imports the reference module itself and runs only when OMNI_REFERENCE_DIR names it."""
 import importlib.util
+import json
 import os
 import sys
 
@@ -9,11 +10,9 @@ import cv2
 import numpy as np
 import pytest
 
-from conftest import REFERENCE_DIR
+from conftest import GOLDEN, REFERENCE_DIR
 from oracle import refport as rp
-from helpers import synth, uniform_img
-
-pytestmark = pytest.mark.reference
+from helpers import PIPE_CASES, load_pipe_case
 
 
 def _load(fname, modname):
@@ -27,49 +26,41 @@ def _load(fname, modname):
 
 
 def test_kmeans_lab_and_assign():
-    ce = _load("02_color_extract.py", "ref_ce")
-    img = synth(300, 400, 5)
-    for K in (4, 8):
-        cv2.setRNGSeed(0)
-        c_ref, l_ref = ce._kmeans_lab(img, K)
-        c = rp.kmeans_lab_centers(img, K)
-        assert np.array_equal(c, c_ref)
-        assert np.array_equal(rp.assign_lab(img, c), l_ref)
-        assert np.array_equal(rp.assign_lab_chunked(img, c, rows=37), l_ref)
-    assert [ce._darkness_rank(n) for n in ("layer_dark", "x_MID", "skin", "Light", "foo")] == \
-           [rp.darkness_rank(n) for n in ("layer_dark", "x_MID", "skin", "Light", "foo")]
+    """02:32-56 in a fresh process (centres, raw labels) and 02:17-23 (layer names by darkness rank -> cluster index) against
+    the centres, labels and palette_by_name.json frozen from the reference on the pipeline cases (K = 4, 4, 8)."""
+    for case in PIPE_CASES:
+        z, meta = load_pipe_case(case)
+        names = meta["names"]
+        c = rp.kmeans_lab_centers(z["resized"], len(names))
+        assert np.array_equal(c, z["centers"]), case
+        assert np.array_equal(rp.assign_lab(z["resized"], c), z["labels"]), case
+        assert np.array_equal(rp.assign_lab_chunked(z["resized"], c, rows=37), z["labels"]), case
+        ranked = sorted(names, key=rp.darkness_rank)
+        assert [ranked.index(n) for n in names] == [meta["palette_by_name"][n]["cluster_index"] for n in names], case
 
 
 def test_assign_labels_rgb():
-    pc = _load("process_colors.py", "ref_pc")
-    img = uniform_img(90, 110, 3)
-    for K in (2, 5, 16):
-        pal = np.random.default_rng(K).integers(0, 256, (K, 3), dtype=np.uint8)
-        assert np.array_equal(rp.assign_labels_rgb(img, pal), pc.assign_labels(img, pal))
+    """process_colors.py:69-77 (int16 wrap) against the label maps the reference CLI saved (K = 5, analyzer and eight palettes)."""
+    z = np.load(os.path.join(GOLDEN, "process_colors.npz"))
+    meta = json.load(open(os.path.join(GOLDEN, "process_colors.json")))
+    rgb = cv2.cvtColor(z["input"], cv2.COLOR_BGR2RGB)
+    for case in ("adaptive5", "analyzer", "eight"):
+        pal = np.array([c["rgb"] for c in meta[case]["palette"]["colors"]], np.uint8)
+        assert np.array_equal(rp.assign_labels_rgb(rgb, pal), z[f"labels_{case}"]), case
 
 
-def test_edge_layer_and_resize(tmp_path):
-    ed = _load("03_edge_detect.py", "ref_ed")
-    rz = _load("01_resize.py", "ref_rz")
-    cfgm = sys.modules["config"]
-    img = synth(260, 380, 9)
-    p = str(tmp_path / "in.png")
-    cv2.imwrite(p, img)
-    for md in (2000, 190, 100):
-        assert np.array_equal(rz.resize_if_needed(p, cfgm.Config(max_dimension=md)), rp.resize_if_needed(img, md))
-    K = 4
-    _, _, masks = rp.color_extract(img, K)
-    names = ["layer_dark", "layer_mid", "layer_skin", "layer_light"]
-    for ks, lo, hi in [(3, 50, 150), (6, 22, 70)]:
-        cfg = cfgm.Config(output_dir=str(tmp_path), color_names=names, edge_kernel_size=ks,
-                          edge_low_threshold=lo, edge_high_threshold=hi)
-        cfg.ensure_output_dirs()
-        for n, m in zip(names, masks):
-            cv2.imwrite(str(tmp_path / n / "mask.png"), m)
-            ed.process_color(n, cfg)
-            e = cv2.imread(str(tmp_path / n / "edges.png"), cv2.IMREAD_GRAYSCALE)
-            assert np.array_equal(e, rp.edge_layer(m, lo, hi, ks))
-        assert ed._ensure_odd(ks) == rp.ensure_odd(ks)
+def test_edge_layer_and_resize():
+    """01_resize.py:7-23 against the reference's resize_if_needed on its 2:1, 3:1, fractional and no-op paths
+    (functions.npz), and 03_edge_detect.py:13-40 against the edge planes its stage 03 wrote for the pipeline cases
+    (blur 3 / 7 / 5, Canny 50/150, 22/70, 100/200)."""
+    f = np.load(os.path.join(GOLDEN, "functions.npz"))
+    for tag in ("rz_2to1", "rz_3to1", "rz_frac", "rz_frac2", "rz_noop"):
+        assert np.array_equal(rp.resize_if_needed(f[tag + "_src"], int(f[tag + "_md"])), f[tag + "_dst"]), tag
+    for case in PIPE_CASES:
+        z, meta = load_pipe_case(case)
+        cfg = meta["config"]
+        for m, e in zip(z["masks"], z["edges"]):
+            assert np.array_equal(rp.edge_layer(m, cfg["edge_low_threshold"], cfg["edge_high_threshold"], cfg["edge_kernel_size"]), e), case
 
 
 def test_skeleton_degree_global_equals_per_component():
@@ -85,6 +76,7 @@ def test_skeleton_degree_global_equals_per_component():
         assert ep.any() or jn.any()
 
 
+@pytest.mark.reference
 def test_stage04_swap_point_with_real_reference(tmp_path):
     """The stage-04 shim (image_processor/04_find_contours.py) replaces ONE module global of the reference's stage 04.
     With the real reference file: the names the shim relies on exist, `vectorize_layer` resolves `thinning_zhangsuen`

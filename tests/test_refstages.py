@@ -1,8 +1,9 @@
-"""Build-container checks (marker `reference`: need /root/reference):
+"""The reference's stage structure:
   * oracle/refstages.py -- the as-shipped CPU baseline bench.py times on the GPU box -- writes the same files as the unmodified
-    reference's pipeline.py run;
+    reference's `pipeline.py --start-step 1 --end-step 3` wrote for the golden pipeline cases (tools/make_golden.py);
   * the drop-in stage scripts copied beside a copy of the reference's pipeline.py are the files its build_steps()/module_path()
-    resolve (INTEGRATION.md, section A), and its own `missing_for_step` bookkeeping accepts the outputs they are expected to write."""
+    resolve (INTEGRATION.md, section A), and its own `missing_for_step` bookkeeping accepts the outputs they are expected to write.
+    This one imports the reference's runner and runs only when OMNI_REFERENCE_DIR names it."""
 import importlib.util
 import json
 import os
@@ -14,12 +15,11 @@ import cv2
 import numpy as np
 import pytest
 
-from helpers import synth
+from conftest import REFERENCE_DIR as REF
+from helpers import PIPE_CASES, load_pipe_case
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = "/root/reference/image_processor"
 DROPIN = os.path.join(ROOT, "omnirevolve-image-processor_b200", "image_processor")
-pytestmark = pytest.mark.reference
 
 
 def _files(outdir, names):
@@ -31,32 +31,28 @@ def _files(outdir, names):
 
 
 def test_refstages_equals_reference_pipeline(tmp_path):
-    img = synth(300, 420, 3)
-    src = tmp_path / "input.png"
-    cv2.imwrite(str(src), img)
     env = dict(os.environ, PYTHONDONTWRITEBYTECODE="1")
-    out_ref = tmp_path / "ref"
-    out_ref.mkdir()
-    r = subprocess.run([sys.executable, os.path.join(REF, "pipeline.py"), str(src), "--output", str(out_ref), "--start-step", "1",
-                        "--end-step", "3"], env=env, stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True)
-    assert r.returncode == 0, r.stdout[-2000:]
-    cfg = json.load(open(out_ref / "config.json"))
-    out_port = tmp_path / "port"
-    out_port.mkdir()
-    cfg2 = dict(cfg, output_dir=str(out_port))
-    (out_port / "config.json").write_text(json.dumps(cfg2))
-    for st in ("01", "02", "03"):
-        r = subprocess.run([sys.executable, os.path.join(ROOT, "oracle", "refstages.py"), st],
-                           env=dict(env, CONFIG_PATH=str(out_port / "config.json")), stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True)
-        assert r.returncode == 0, r.stdout[-2000:]
-    names = cfg["color_names"]
-    a, b = _files(str(out_ref), names), _files(str(out_port), names)
-    assert np.array_equal(a[0], b[0])
-    for x, y in zip(a[1] + a[2], b[1] + b[2]):
-        assert np.array_equal(x, y)
-    assert np.array_equal(a[3], b[3]) and a[4] == b[4]
+    for case in PIPE_CASES:
+        z, meta = load_pipe_case(case)
+        src = tmp_path / f"{case}.png"
+        cv2.imwrite(str(src), z["input"])
+        out_port = tmp_path / case
+        out_port.mkdir()
+        cfg = dict(meta["config"], input_image=str(src), output_dir=str(out_port))
+        (out_port / "config.json").write_text(json.dumps(cfg))
+        for st in ("01", "02", "03"):
+            r = subprocess.run([sys.executable, os.path.join(ROOT, "oracle", "refstages.py"), st],
+                               env=dict(env, CONFIG_PATH=str(out_port / "config.json")), stdout=subprocess.PIPE,
+                               stderr=subprocess.STDOUT, text=True)
+            assert r.returncode == 0, r.stdout[-2000:]
+        resized, masks, edges, comp, palette = _files(str(out_port), meta["names"])
+        assert np.array_equal(resized, z["resized"]), case
+        for i, n in enumerate(meta["names"]):
+            assert np.array_equal(masks[i], z["masks"][i]) and np.array_equal(edges[i], z["edges"][i]), (case, n)
+        assert np.array_equal(comp, z["composite"]) and palette == meta["palette_by_name"], case
 
 
+@pytest.mark.reference
 def test_reference_pipeline_resolves_the_dropins(tmp_path):
     """Copy the reference's runner + config module and OUR stage scripts into one directory, as INTEGRATION.md A says, and ask
     the runner itself which files it would launch and which outputs it waits for."""
