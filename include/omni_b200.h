@@ -256,6 +256,26 @@ int omni_skeleton_degree(omni_ctx *ctx, const uint8_t *d_skel, int K, int h, int
                          uint8_t *d_deg, size_t d_plane_stride, size_t dpitch,
                          uint8_t *d_nodes, size_t n_plane_stride, size_t npitch, void *stream);
 
+/* ---- stage 04: 04_find_contours.py:101-205  trace_centerlines(skel, layer) ------------------------ */
+/* K skeleton planes (a pixel > 0 is foreground, `S = (skel > 0)`, 04:103), plane p at d_skel + p*plane_stride, rows pitch
+ * bytes apart.  Replaces the whole function: cv2.connectedComponentsWithStats(S, connectivity=8) (04:108; same labels, same
+ * stats), the per-component degree / endpoint / junction maps (04:117-125) and the walk (04:126-200: open paths from the
+ * endpoints, then the cycles, same guards, same closing point), one component per CTA.  The polylines are the reference's:
+ * same points in the same order.
+ * The output size is found on the device, so the call SYNCHRONISES the stream.  h_plane_info (optional, 4*K int64): per plane
+ * [total_fg, components, polylines, points].  The results stay in the ctx until the next omni_trace_centerlines /
+ * omni_host_trace_centerlines call on it; omni_trace_results copies them out. */
+int omni_trace_centerlines(omni_ctx *ctx, const uint8_t *d_skel, int K, int h, int w, size_t plane_stride, size_t pitch,
+                           int64_t *h_plane_info, void *stream);
+/* Host-buffer form: h_skel is copied in, then as omni_trace_centerlines. */
+int omni_host_trace_centerlines(omni_ctx *ctx, const uint8_t *h_skel, int K, int h, int w, size_t plane_stride, size_t pitch,
+                                int64_t *h_plane_info);
+/* Copies the result of the last trace into caller buffers (host or device memory; any may be NULL) and returns when they hold it:
+ * h_points: int32 [points][2] = (x, y) of every polyline, planes in order, components in label order (cv2's), polylines in the
+ * reference's order; h_path_len: int32 [polylines], the number of points of each; h_comp: int32 [components][6] = cv2's stats row
+ * (left, top, width, height, area) plus the number of polylines of the component.  Sizes: the totals of h_plane_info. */
+int omni_trace_results(omni_ctx *ctx, int32_t *h_points, int32_t *h_path_len, int32_t *h_comp);
+
 /* Diagnostics of the last omni_edges / omni_color_edge call on this ctx: number of global
  * hysteresis passes that were needed (>= 1). */
 int omni_last_hysteresis_passes(omni_ctx *ctx);

@@ -1023,6 +1023,36 @@ extern "C" int omni_skeleton_degree(omni_ctx *ctx, const uint8_t *d_skel, int K,
     return OMNI_OK;
 }
 
+// ---- stage 04: trace_centerlines (trace.cu) ----------------------------------------------------------------
+extern "C" int omni_trace_centerlines(omni_ctx *ctx, const uint8_t *d_skel, int K, int h, int w, size_t plane_stride, size_t pitch,
+                                      int64_t *h_plane_info, void *stream)
+{
+    OMNI_TRY(set_device(ctx));
+    OMNI_REQUIRE(d_skel && K >= 1 && K <= OMNI_MAX_K && h > 0 && w > 0, "omni_trace_centerlines: bad arguments");
+    OMNI_REQUIRE(pitch >= (size_t)w && (K == 1 || plane_stride >= pitch * (h - 1) + w), "omni_trace_centerlines: pitch smaller than a row");
+    OMNI_REQUIRE((long long)((w + 1) / 2) * ((h + 1) / 2) * K < INT32_MAX, "omni_trace_centerlines: %d planes of %d x %d are too large", K, w, h);
+    return trace_run(ctx, d_skel, K, h, w, plane_stride, pitch, h_plane_info, (cudaStream_t)stream);
+}
+
+extern "C" int omni_host_trace_centerlines(omni_ctx *ctx, const uint8_t *h_skel, int K, int h, int w, size_t plane_stride, size_t pitch,
+                                           int64_t *h_plane_info)
+{
+    OMNI_TRY(set_device(ctx));
+    OMNI_REQUIRE(h_skel && K >= 1 && K <= OMNI_MAX_K && h > 0 && w > 0 && pitch >= (size_t)w, "omni_host_trace_centerlines: bad arguments");
+    size_t dp = pad16((size_t)w), dplane = dp * h;
+    OMNI_TRY(omni_ws_reserve(ctx, 3, pad16(dplane * K)));
+    u8 *d = (u8 *)ctx->ws[3];
+    for (int k = 0; k < K; k++)
+        OMNI_CUDA(cudaMemcpy2DAsync(d + k * dplane, dp, h_skel + k * plane_stride, pitch, (size_t)w, h, cudaMemcpyHostToDevice, ctx->stream));
+    return omni_trace_centerlines(ctx, d, K, h, w, dplane, dp, h_plane_info, ctx->stream);
+}
+
+extern "C" int omni_trace_results(omni_ctx *ctx, int32_t *h_points, int32_t *h_path_len, int32_t *h_comp)
+{
+    OMNI_TRY(set_device(ctx));
+    return trace_results(ctx, h_points, h_path_len, h_comp);
+}
+
 extern "C" int omni_host_color_edge(omni_ctx *ctx, const uint8_t *h_bgr, int h, int w, size_t pitch,
                                     const float *h_centers, int K, const uint8_t *h_lut, const omni_edge_params *prm,
                                     uint8_t *h_labels, size_t lpitch,

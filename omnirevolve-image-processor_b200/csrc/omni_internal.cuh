@@ -57,12 +57,12 @@ struct ResizeTab {
     ResizeTabDev dev{};
 };
 
-#define OMNI_WS_SLOTS 7
+#define OMNI_WS_SLOTS 11
 struct omni_ctx {
     int device = 0;
     int fast = 1;
     // grow-only device scratch
-    void *ws[OMNI_WS_SLOTS] = {};          // 0-2 generic planes, 3 host staging, 4 bit-planes, 5 misc, 6 edge run lists
+    void *ws[OMNI_WS_SLOTS] = {};          // 0-2 generic planes, 3 host staging, 4 bit-planes, 5 misc, 6 edge run lists, 7-10 trace.cu
     size_t ws_bytes[OMNI_WS_SLOTS] = {};
     int *d_flags = nullptr;          // 64 ints of device flags / counters
     unsigned long long *d_counts = nullptr;   // 4*OMNI_MAX_K counters
@@ -120,6 +120,11 @@ struct omni_ctx {
     size_t pk_counts_cap = 0;                  // groups of 3 * OMNI_MAX_K counts
     int pipeline = 1;                          // fused colour+edge call: 1 = sparse generation (label_pipe.cu), 0 = dense generation
     u8 *d_rgb_boxes = nullptr;                 // exact Lab box of every 4x4x4 RGB cell (centre-independent, built on first use)             // co-resident CTAs of the cooperative hysteresis kernel (0 = not queried yet)
+    // result of the last omni_trace_centerlines call: polylines in ws[10], sizes and per-component rows on the host
+    int trace_valid = 0, trace_K = 0;
+    long long trace_points = 0, trace_paths = 0;
+    std::vector<long long> trace_info;         // per plane: total_fg, components, polylines, points
+    std::vector<int32_t> trace_comp;           // per component: left, top, width, height, area, polylines
 };
 
 // Brackets one kernel launch: counts it and, when profiling is on, records a CUDA event pair on the
@@ -132,6 +137,10 @@ struct KScope {
 #define OMNI_LAUNCH(ctx, st, name, expr) do { KScope ks__(ctx, name, st); OMNI_CUDA(expr); } while (0)
 
 int omni_ws_reserve(omni_ctx *ctx, int slot, size_t bytes);
+// stage 04 trace_centerlines (trace.cu): run on K planes (synchronises st), then copy the results out
+int trace_run(omni_ctx *ctx, const u8 *d_skel, int K, int h, int w, size_t plane_stride, size_t pitch, int64_t *h_info,
+              cudaStream_t st);
+int trace_results(omni_ctx *ctx, int32_t *points, int32_t *path_len, int32_t *comp);
 const ResizeTab *omni_get_resize_tab(omni_ctx *ctx, int sh, int sw, int dh, int dw, cudaStream_t st);
 void omni_build_se(int shape_ellipse, int k, MorphSE *se);
 int omni_gauss_weights(int k, BlurParams *bp);

@@ -1,11 +1,10 @@
-# 04_find_contours.py -- drop-in SHIM for the reference's stage 04.  The data-parallel parts of the stage run on the GPU:
-# `thinning_zhangsuen` (04_find_contours.py:35-99 of the reference, Zhang-Suen thinning of the edge planes) and the degree /
-# endpoint / junction maps `trace_centerlines` needs (04:117-125; one pass over the skeleton instead of a full-image filter2D per
-# connected component).  The walk along the skeleton is sequential by construction: omni_b200.contours.trace_centerlines keeps it
-# step for step (same polylines, same order, same log lines; tests/golden/trace.npz is frozen from the reference) but confines
-# every component to its bounding box.  Everything else is the reference's own code: rename the reference's file to
-# `04_find_contours_ref.py` (same directory) and put this file in its place -- it loads the original module, swaps the two
-# functions and runs the original `vectorize_all`, so contours.pkl and the log are the reference's.
+# 04_find_contours.py -- drop-in SHIM for the reference's stage 04.  Both GPU-backed steps come from omni_b200.contours:
+# `thinning_zhangsuen` (04_find_contours.py:35-99 of the reference, Zhang-Suen thinning of the edge planes) and
+# `trace_centerlines` (04:101-205): connected components, degree maps and the walk along the skeleton in one call
+# (omni_trace_centerlines), one component per CTA -- same polylines, same order, same log lines except the time-driven
+# "visited" lines (tests/golden/trace.npz is frozen from the reference).  Everything else is the reference's own code: rename
+# the reference's file to `04_find_contours_ref.py` (same directory) and put this file in its place -- it loads the original
+# module, swaps the two functions and runs the original `vectorize_all`, so contours.pkl and the log are the reference's.
 import importlib.util
 import os
 import sys

@@ -26,6 +26,7 @@ EXPORTS = [
     "omni_set_table_cache", "omni_host_edges_composite", "omni_color_edge_packed", "omni_host_color_edge_packed",
     "omni_workspace_bytes", "omni_ctx_reserve", "omni_set_assume_binary_masks", "omni_kmeans_lab",
     "omni_thin_zhangsuen_packed", "omni_set_host_bands", "omni_last_band_resends",
+    "omni_trace_centerlines", "omni_host_trace_centerlines", "omni_trace_results",
 ]
 
 
@@ -97,6 +98,9 @@ def lib():
         "omni_color_edge_packed": ([vp, u8p, i, sz, i, i, sz, f32p, i, hu8, epp, u8p, sz, sz, u8p, sz, sz, i, i64p, vp], i),
         "omni_host_color_edge_packed": ([vp, u8p, i, sz, i, i, sz, f32p, i, hu8, epp, u8p, sz, sz, u8p, sz, sz, i, i64p], i),
         "omni_swatch_masks": ([vp, u8p, i, i, sz, i32p, i, i, u8p, sz, sz, i32p, vp], i),
+        "omni_trace_centerlines": ([vp, u8p, i, i, i, sz, sz, i64p, vp], i),
+        "omni_host_trace_centerlines": ([vp, u8p, i, i, i, sz, sz, i64p], i),
+        "omni_trace_results": ([vp, vp, vp, vp], i),
     }
     for name, (args, res) in sig.items():
         fn = getattr(L, name)

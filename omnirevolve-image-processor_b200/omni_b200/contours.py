@@ -1,17 +1,19 @@
-"""Stage 04, first step: the reference's `thinning_zhangsuen` (04_find_contours.py:35-99) on the GPU.
+"""Stage 04 of the reference (04_find_contours.py) on the GPU: `thinning_zhangsuen` (04:35-99) and `trace_centerlines`
+(04:101-205).
 
-Only the data-parallel part of stage 04 lives here (SURVEY.md 8f rank 1): the skeleton the reference computes with
-NumPy shifts in ~10^2 s per layer comes out of the bit-plane kernel `omni_thin_zhangsuen` in well under a
-millisecond.  `trace_centerlines` (04:101-205) walks the skeleton sequentially and stays the reference's own code;
-it consumes the array returned here unchanged.
+The skeleton the reference computes with NumPy shifts in ~10^2 s per layer comes out of the bit-plane kernel
+`omni_thin_zhangsuen` in well under a millisecond.  The walk of `trace_centerlines` is sequential within one connected
+component, but the components are independent: `omni_trace_centerlines` labels them on the device (cv2's numbering and
+stats) and walks every component in its own CTA, step for step as the reference does.
 
     thinning_zhangsuen(bin_0_255, layer)      same signature, same result, same progress lines (04:37-95)
     thin_layers(planes)                        all K edge planes in one call (what a fused stage 03 -> 04 hand-off uses)
-    trace_centerlines(skel_0_255, layer)      same signature, same polylines in the same order, same progress lines (04:101-205);
-                                               the degree / endpoint / junction maps come from ONE GPU pass over the skeleton
-                                               (omni_skeleton_degree) and every component is handled inside its bounding box --
-                                               the reference recomputes `labels == comp_id` and a filter2D over the WHOLE image
-                                               per component (04:113-125), which is the stage's O(components x pixels) term
+    trace_centerlines(skel_0_255, layer)      same signature, same polylines in the same order, same progress lines
+                                               (04:101-205) except the time-driven "visited n/m px" lines; one GPU call
+    trace_layers(skels, names)                 all K layers in one GPU call, each layer's log lines in turn
+    trace_centerlines(skel, layer, maps=...)   the host walk (a Python restatement of 04:126-200 that takes the degree /
+                                               endpoint / junction maps of the whole skeleton and confines every component to
+                                               its bounding box): the reference the GPU tracer is tested against
 """
 from __future__ import annotations
 
@@ -73,13 +75,48 @@ def skeleton_degree(skel_0_255: np.ndarray):
 NEIGH8 = [(-1, -1), (0, -1), (1, -1), (-1, 0), (1, 0), (-1, 1), (0, 1), (1, 1)]          # 04_find_contours.py:12 (the visiting order)
 
 
+def _log_trace(r, layer: str, dt: float):
+    """The log lines of 04:104-205 for one plane from the GPU result (the seconds are the call's, shared over the components)."""
+    if r.total_fg == 0:
+        print(f"[{layer}] Trace: empty skeleton.", flush=True)
+        return []
+    n = len(r.stats)
+    print(f"[{layer}] Trace: fg={r.total_fg} px | components={n}", flush=True)
+    done = so_far = 0
+    for i, (area, npl) in enumerate(zip(r.stats[:, 4].tolist(), r.polylines.tolist()), 1):
+        done += area
+        so_far += npl
+        print(f"[{layer}]  \u2022 Component {i}/{n}: pixels={area}", flush=True)
+        print(f"[{layer}]  \u2022 Component {i} done in {dt / n:.2f}s, polylines so far: {so_far}", flush=True)
+        print(f"[{layer}]  \u2022 Progress: components_fg {done}/{r.total_fg} px ({100.0 * done / r.total_fg:4.1f}%)", flush=True)
+    print(f"[{layer}] Trace done: {len(r.paths)} polylines in {dt:.2f}s", flush=True)
+    return r.paths
+
+
+def trace_layers(skels: np.ndarray, names):
+    """trace_centerlines of K skeleton planes [K,H,W] in ONE GPU call; prints each layer's log lines in turn (the seconds are the
+    call's time shared over the layers) and returns the K polyline lists."""
+    t0 = time.perf_counter()
+    res = get_engine().host_trace_centerlines(skels)
+    dt = (time.perf_counter() - t0) / max(1, len(res))
+    return [_log_trace(r, name, dt) for r, name in zip(res, names)]
+
+
 def trace_centerlines(skel_0_255: np.ndarray, layer: str, maps=None):
-    """Drop-in for 04_find_contours.py:101-205.  The walk itself is sequential by construction and is kept step for step (start
-    pixels in row-major order, NEIGH8 neighbour order, the same guards); what changes is where its inputs come from:
-    `maps` = (deg, endpoints, junctions) of the whole skeleton, by default one omni_skeleton_degree call -- on the pixels of a
-    component they equal the reference's per-component maps, because the 8-neighbours of a component pixel belong to that
-    component -- and each component lives in its bounding box (cv2.connectedComponentsWithStats, same labels).  The time-driven
-    "visited n/m px" lines appear when 1.5 s have passed, as in the reference, but are only looked at every 1024 steps."""
+    """Drop-in for 04_find_contours.py:101-205: the reference's polylines in the reference's order, the same log lines.
+    maps=None: one GPU call (omni_trace_centerlines).  maps=(deg, endpoints, junctions) of the whole skeleton: the host walk."""
+    if maps is None:
+        return trace_layers(np.asarray(skel_0_255)[None], [layer])[0]
+    return _trace_host(skel_0_255, layer, maps)
+
+
+def _trace_host(skel_0_255: np.ndarray, layer: str, maps):
+    """The host walk, kept step for step (start pixels in row-major order, NEIGH8 neighbour order, the same guards); what
+    changes against the reference is where its inputs come from: `maps` = (deg, endpoints, junctions) of the whole skeleton --
+    on the pixels of a component they equal the reference's per-component maps, because the 8-neighbours of a component pixel
+    belong to that component -- and each component lives in its bounding box (cv2.connectedComponentsWithStats, same labels).
+    The time-driven "visited n/m px" lines appear when 1.5 s have passed, as in the reference, but are only looked at every
+    1024 steps."""
     t0 = time.perf_counter()
     S = (skel_0_255 > 0).astype(np.uint8)
     total_fg = int(S.sum())
@@ -88,8 +125,6 @@ def trace_centerlines(skel_0_255: np.ndarray, layer: str, maps=None):
         return []
     num, labels, stats, _c = cv2.connectedComponentsWithStats(S, connectivity=8)
     print(f"[{layer}] Trace: fg={total_fg} px | components={num-1}", flush=True)
-    if maps is None:
-        maps = skeleton_degree(skel_0_255)
     _deg_all, ep_all, jn_all = maps
     paths = []
     comp_fg_done = 0

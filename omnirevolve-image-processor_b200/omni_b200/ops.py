@@ -59,6 +59,15 @@ class EdgeConfig:
                                self.ensure_odd(self.ksize), float(self.low), float(self.high))
 
 
+@dataclass
+class TraceResult:
+    """trace_centerlines of one skeleton plane (04_find_contours.py:101-205)."""
+    paths: list            # int32 (n,1,2) arrays of (x, y): the reference's polylines in its order
+    stats: np.ndarray      # int32 [components, 5]: cv2.connectedComponentsWithStats' stats rows 1.. (left, top, width, height, area)
+    polylines: np.ndarray  # int32 [components]: polylines of each component
+    total_fg: int          # skeleton pixels of the plane
+
+
 def _f32p(a):
     return a.ctypes.data_as(C.POINTER(C.c_float))
 
@@ -411,6 +420,49 @@ class Engine:
             self._h, planes.ctypes.data, K, h, w, planes.strides[0], planes.strides[1], int(max_iter),
             out.ctypes.data, out.strides[0], out.strides[1], removed.ctypes.data_as(i32p), iters.ctypes.data_as(i32p)))
         return out, removed[:, :max_iter], iters
+
+    # ---- stage 04: trace_centerlines ----------------------------------------------------------------
+    def trace_centerlines(self, skel: torch.Tensor) -> list["TraceResult"]:
+        """04_find_contours.py:101-205 on K skeleton planes [K,H,W] u8 (> 0 = foreground): per plane a TraceResult (the
+        reference's polylines in its order, cv2's component stats).  Synchronises the current stream."""
+        _check_planes(skel)
+        K, h, w = skel.shape
+        info = np.zeros((K, 4), np.int64)
+        capi.check(self._L.omni_trace_centerlines(self._h, skel.data_ptr(), K, h, w, skel.stride(0), skel.stride(1),
+                                                  info.ctypes.data_as(C.POINTER(C.c_int64)), self._stream()))
+        return self._trace_results(info)
+
+    def host_trace_centerlines(self, skel: np.ndarray) -> list["TraceResult"]:
+        """Host-buffer form of trace_centerlines: NumPy [K,H,W] or [H,W] (> 0 = foreground; ctypes + NumPy only)."""
+        a = np.asarray(skel)
+        if a.ndim == 2:
+            a = a[None]
+        if a.ndim != 3:
+            raise ValueError("expected skeleton planes [K,H,W] or one [H,W]")
+        if a.dtype != np.uint8:
+            a = (a > 0).astype(np.uint8)
+        elif a.strides[2] != 1 or a.strides[1] < a.shape[2] or a.strides[0] < 0 or a.strides[1] < 0:
+            a = np.ascontiguousarray(a)
+        K, h, w = a.shape
+        info = np.zeros((K, 4), np.int64)
+        capi.check(self._L.omni_host_trace_centerlines(self._h, a.ctypes.data, K, h, w, a.strides[0], a.strides[1],
+                                                       info.ctypes.data_as(C.POINTER(C.c_int64))))
+        return self._trace_results(info)
+
+    def _trace_results(self, info: np.ndarray) -> list["TraceResult"]:
+        n_comp, n_paths, n_pts = (int(v) for v in info[:, 1:].sum(axis=0))
+        pts = np.empty((n_pts, 2), np.int32)
+        lens = np.empty(n_paths, np.int32)
+        comp = np.empty((n_comp, 6), np.int32)
+        capi.check(self._L.omni_trace_results(self._h, pts.ctypes.data, lens.ctypes.data, comp.ctypes.data))
+        out, c0, l0, p0 = [], 0, 0, 0
+        for total_fg, nc, npath, npt in info.tolist():
+            ln = lens[l0:l0 + npath]
+            pl = pts[p0:p0 + npt].reshape(-1, 1, 2)
+            paths = np.split(pl, np.cumsum(ln[:-1])) if npath else []
+            out.append(TraceResult(paths, comp[c0:c0 + nc, :5], comp[c0:c0 + nc, 5], int(total_fg)))
+            c0, l0, p0 = c0 + nc, l0 + npath, p0 + npt
+        return out
 
     def last_hysteresis_passes(self) -> int:
         return int(self._L.omni_last_hysteresis_passes(self._h))
