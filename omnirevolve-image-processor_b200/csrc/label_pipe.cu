@@ -7,15 +7,16 @@
 //                      (02_color_extract.py:35-36,53-55,121-127; the same exact table-driven assignment as fk_assign_rgbcell, but a
 //                      lane owns 8 consecutive pixels -- three 8-byte shared-memory loads instead of 24 byte loads -- and there are
 //                      no per-plane stores and no __match_any: 4 slice words per 32 pixels come out of a 4x4 byte transpose)
-//   fk_label_open      RECT-3 OPEN of all K one-hot planes at once, in the label domain (02:152):
+//   fk_open_morph      a CTA stages the label slices of one strip in shared memory (bulk copies, mbarrier completion) and computes
+//                      the RECT-3 OPEN of all K one-hot planes at once, in the label domain (02:152):
 //                        erode_k  = [label == k] & U        U  = "the 3x3 neighbourhood (inside the image) has one label"
 //                        open_k   = [label == k] & Od       Od = dilate3(U)     (a pixel next to a uniform pixel q has q's label)
-//                      so the first two steps of the chain cost ONE plane (Od) instead of K
-//   fk_morph_lab       per plane k: open_k = Od & [label == k] from the slices on the fly, then the remaining steps (02:153 RECT-3
-//                      close -> mask BYTES; 03:23-30 ELLIPSE-3 open/close -> bit-plane M2) on 32-bit words: lanes are adjacent word
-//                      columns, the neighbour bits of a step come from two warp shuffles (ALU pipe: 2 LOP3 + 2 SHF per step and
-//                      32 pixels instead of 4 + 4 on a 64-bit window); 30 owned columns + a halo lane on each side per warp.
-//                      Classifies its tiles for the sparse edge kernel (edges3.cu) like fk_morph does.
+//                      so the first two steps of the chain cost ONE plane (Od, kept in shared memory) instead of K.  Then one warp
+//                      per plane k: open_k = Od & [label == k], the remaining steps (02:153 RECT-3 close -> mask BYTES; 03:23-30
+//                      ELLIPSE-3 open/close -> bit-plane M2) on 32-bit words: lanes are adjacent word columns, the neighbour bits
+//                      of a step come from two warp shuffles (ALU pipe: 2 LOP3 + 2 SHF per step and 32 pixels instead of 4 + 4 on
+//                      a 64-bit window); 30 owned columns + a halo lane on each side per warp.  Classifies its tiles for the
+//                      sparse edge kernel (edges3.cu) like fk_morph does.
 //   fk_edges3_simd<sparse> + fk_hysteresis as before.
 //
 // Reference call sites are relative to /root/reference/image_processor/.  Bit-exactness against the oracle is checked by the same
@@ -324,88 +325,29 @@ __global__ void __launch_bounds__(RA_THREADS, 1) fk_assign_slices(const u8 *__re
 }
 
 // ------------------------------------------------------------------------------------------------
-// fk_label_open: Od = dilate3(U), one bit-plane per frame.  A lane owns a word column and walks down a strip; a warp covers 30
-// owned columns + a halo lane on each side (the dilation needs U of the neighbouring words).  Per label row r:
-//   dh(r) = "differs from the left or right neighbour",  dv(r) = "differs from the pixel above"      (bit-slice XORs)
-//   U(r-1) = ~(dh(r-2) | dh(r-1) | dh(r) | dv(r-1) | dv(r))         (neighbours outside the image are ignored, as cv2.erode does)
-//   Od(r-2) = hU(r-3) | hU(r-2) | hU(r-1),  hU = U | U << 1 | U >> 1                                    (cv2.dilate: outside = 0)
+// fk_open_morph: the label-domain RECT-3 open and the rest of the morphology chain in one kernel.  A CTA is one frame, one strip
+// of TR rows and one group of 30 word columns, with one warp per plane of a group of at most OM_PMAX planes of that frame.  The
+// lanes of a warp cover the word columns c0-1 .. c0+30 and lanes 1..30 own theirs; a halo lane's word is wrong in one more outer
+// bit per step, never in the bit its owned neighbour reads.
+//   1. Staging: thread 0 issues one cp.async.bulk per label row (the 4 slice words of the columns c0-2 .. c0+31 are 34 adjacent
+//      uint4, 544 B) for all rows [y0 - N - EXT - 2, y1 + N + EXT + 2) of the strip at once, one mbarrier per OM_CHUNK rows.
+//      Columns and rows outside the image are zeros in shared memory.  The strip is fetched once per CTA, not once per plane.
+//   2. Od = dilate3(U), once per CTA, the warps splitting the rows.  Per label row r:
+//        dh(r) = "differs from the left or right neighbour",  dv(r) = "differs from the pixel above"      (bit-slice XORs)
+//        U(r-1) = ~(dh(r-2) | dh(r-1) | dh(r) | dv(r-1) | dv(r))       (neighbours outside the image are ignored, as cv2.erode does)
+//        Od(r-2) = hU(r-3) | hU(r-2) | hU(r-1),  hU = U | U << 1 | U >> 1                                  (cv2.dilate: outside = 0)
+//      Lanes 0 and 31 also track U of the staged columns c0-2 / c0+31, so that Od is exact in all 32 lanes.
+//   3. Per plane k: open_k = Od & [label == k] from shared memory, then the remaining steps on 32-bit words with the neighbour
+//      bits from warp shuffles: 02:153 RECT-3 close -> mask bytes, 03:23-30 ELLIPSE-3 open / close -> bit-plane M2; the tiles are
+//      classified and the run lists of the sparse edge kernel written as fk_morph (fast_kernels.cu) does.
 // ------------------------------------------------------------------------------------------------
-#define LO_WARPS 4
-#define LP_COLS 30                        // owned word columns per warp (fk_label_open, fk_morph_lab)
-#define LO_ROWS 8                         // rows per strip (short strips: the kernel is latency-bound, it needs many warps)
+#define LP_COLS 30                        // owned word columns per warp
+#define OM_SCOLS 34                       // staged word columns per row: c0-2 .. c0+31
+#define OM_CHUNK 8                        // staged rows per mbarrier
+#ifndef OM_PMAX
+#define OM_PMAX 8                         // plane-warps per CTA, at most
+#endif
 
-__global__ void __launch_bounds__(LO_WARPS * 32) fk_label_open(const uint4 *__restrict__ slices, int ws, size_t plane, int h, int w, int nf,
-                                                               u32 *__restrict__ od_out, int strips, int wcols)
-{
-    const int lane = threadIdx.x & 31;
-    const long long gw = (long long)blockIdx.x * LO_WARPS + (threadIdx.x >> 5);
-    const long long per_f = (long long)strips * wcols;
-    if (gw >= per_f * nf) return;
-    const int f = (int)(gw / per_f);
-    const int rem = (int)(gw - (long long)f * per_f);
-    const int strip = rem / wcols, wx = rem - strip * wcols;
-    const int ww = (w + 31) >> 5;
-    const int c = wx * LP_COLS - 1 + lane;
-    const bool inimg = c >= 0 && c < ww;
-    const bool owned = inimg && lane >= 1 && lane <= LP_COLS;
-    const u32 cm = inimg ? range_mask(32 * c, w) : 0u;
-    const u32 lfix = (c == 0) ? 1u : 0u;                                   // pixel 0 has no left neighbour
-    const u32 rfix = (c == ww - 1) ? (1u << ((w - 1) & 31)) : 0u;          // pixel w-1 has no right neighbour
-    const uint4 *sl = slices + (size_t)f * plane;           // uint4 per word column: the 4 slice words
-    u32 *od = od_out + (size_t)f * plane;
-    const int ys = strip * LO_ROWS, ye = min(h, ys + LO_ROWS);
-    u32 sp[4] = {0u, 0u, 0u, 0u}, dh1 = 0u, dh2 = 0u, dv1 = 0u, hu2 = 0u, hu3 = 0u;
-    u32 ns[4], ne[4];                                                      // slices of the next row (loaded one row ahead)
-    auto fetch = [&](const int r) {
-        const bool rin = r >= 0 && r < h;
-        uint4 v = make_uint4(0u, 0u, 0u, 0u), ev = v;
-        if (rin) {
-            const uint4 *row = sl + (size_t)r * ws;
-            if (inimg) v = __ldg(row + c);
-            if (lane == 0 && c - 1 >= 0 && c - 1 < ww) ev = __ldg(row + c - 1);
-            if (lane == 31 && c + 1 >= 0 && c + 1 < ww) ev = __ldg(row + c + 1);
-        }
-        ns[0] = v.x; ns[1] = v.y; ns[2] = v.z; ns[3] = v.w;
-        ne[0] = ev.x; ne[1] = ev.y; ne[2] = ev.z; ne[3] = ev.w;
-    };
-    fetch(ys - 2);
-    for (int r = ys - 2; r < ye + 2; r++) {
-        u32 s[4], e[4];
-#pragma unroll
-        for (int b = 0; b < 4; b++) { s[b] = ns[b]; e[b] = ne[b]; }
-        fetch(r + 1);
-        const bool rin = r >= 0 && r < h;
-        u32 dl = 0u, dr = 0u, dv = 0u;
-#pragma unroll
-        for (int b = 0; b < 4; b++) {
-            const u32 m = s[b];
-            u32 l = __shfl_up_sync(0xffffffffu, m, 1), rr = __shfl_down_sync(0xffffffffu, m, 1);
-            if (lane == 0) l = e[b];
-            if (lane == 31) rr = e[b];
-            dl |= m ^ __funnelshift_l(l, m, 1);
-            dr |= m ^ __funnelshift_r(m, rr, 1);
-            dv |= m ^ sp[b];
-            sp[b] = m;
-        }
-        dl &= ~lfix; dr &= ~rfix;
-        const u32 dh0 = rin ? (dl | dr) : 0u;
-        const u32 dv0 = (rin && r > 0) ? dv : 0u;
-        const bool yin = r - 1 >= 0 && r - 1 < h;
-        const u32 U = yin ? (~(dh2 | dh1 | dh0 | dv1 | dv0) & cm) : 0u;
-        const u32 l = __shfl_up_sync(0xffffffffu, U, 1), rr = __shfl_down_sync(0xffffffffu, U, 1);
-        const u32 hu1 = U | __funnelshift_l(l, U, 1) | __funnelshift_r(U, rr, 1);
-        const int z = r - 2;
-        if (owned && z >= ys && z < ye) od[(size_t)z * ws + c] = (hu3 | hu2 | hu1) & cm;
-        hu3 = hu2; hu2 = hu1; dh2 = dh1; dh1 = dh0; dv1 = dv0;
-    }
-}
-
-// ------------------------------------------------------------------------------------------------
-// fk_morph_lab: the chain after the label-domain open for plane blockIdx.z, on 32-bit words with shuffled neighbour bits.
-// Structure and outputs are fk_morph's (fast_kernels.cu): a strip of TR rows per warp, steps lagging each other by one row in
-// registers, mask bytes tapped after the RECT close, final bit-plane M2 + run lists / dead-tile zeros for the sparse edge kernel.
-// A halo lane's word is wrong in one more outer bit per step, never in the bit its owned neighbour reads.
-// ------------------------------------------------------------------------------------------------
 template <int OP>
 __device__ __forceinline__ u32 step32(const u32 u, const u32 m, const u32 d)
 {
@@ -456,63 +398,146 @@ struct MorphChain32 {
     }
 };
 
-#ifndef ML_ORDER
-#define ML_ORDER 1
-#endif
-#ifndef ML_MINB
-#define ML_MINB 1
-#endif
-// RUNS = false: masks only (stage 02 on its own): no final bit-plane, no tile classification.  masks == NULL: no mask bytes
-// (packed outputs); tap_bits != NULL: the mask as a bit-plane.
-template <u32 CODE, int TAP, int TR, bool RUNS>
-__global__ void __launch_bounds__(128, ML_MINB) fk_morph_lab(const uint4 *__restrict__ slices, const u32 *__restrict__ od, u32 *__restrict__ out_bits, int ws,
-                                                    size_t plane, int h, int w, int K, u8 *__restrict__ masks, size_t mstride, size_t mpitch,
-                                                    int aligned16, u32 *__restrict__ tap_bits, int wcols, int strips, int n_planes, long long n_units,
-                                                    const __grid_constant__ MorphRuns R)
+// shared-memory layout of fk_open_morph: [staged slice rows RS][34] uint4 | Od rows [RO + 1][32] u32
+template <u32 CODE, int TR, bool RUNS>
+struct OmLayout {
+    static constexpr int N = code_len(CODE), EXT = RUNS ? 2 : 0;
+    static constexpr int RS = TR + 2 * (N + EXT + 2);                 // staged label rows, at most
+    static constexpr int RO = TR + 2 * (N + EXT);                     // Od rows, at most (+ 1: the chain fetches one row ahead)
+    static constexpr int NBAR = (RS + OM_CHUNK - 1) / OM_CHUNK;
+    static constexpr int TILES = TR / ET_R;
+    static constexpr size_t OFF_OD = (size_t)RS * OM_SCOLS * sizeof(uint4);
+    static constexpr size_t bytes() { return OFF_OD + (size_t)(RO + 1) * 32 * sizeof(u32); }
+};
+
+__device__ __forceinline__ void om_wait(u32 bar)
 {
-    constexpr int N = code_len(CODE);
-    constexpr int EXT = RUNS ? 2 : 0;
-    constexpr int TILES = TR / ET_R;
+    u32 done = 0;
+    while (!done)
+        asm volatile("{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], 0;\n\tselp.u32 %0, 1, 0, p;\n\t}"
+                     : "=r"(done) : "r"(bar) : "memory");
+}
+
+// RUNS = false: masks only (stage 02 on its own): no final bit-plane, no tile classification.  masks == NULL: no mask bytes
+// (packed outputs); tap_bits != NULL: the mask as a bit-plane.  blockDim.x = 32 P; grid = column groups x planes groups x frames
+// x strips, column groups fastest (the planes of a strip run together, strips top-down).
+template <u32 CODE, int TAP, int TR, bool RUNS>
+__global__ void __launch_bounds__(OM_PMAX * 32) fk_open_morph(const uint4 *__restrict__ slices, u32 *__restrict__ out_bits, int ws, size_t plane,
+                                                             int h, int w, int K, int P, int groups, int nf, u8 *__restrict__ masks,
+                                                             size_t mstride, size_t mpitch, int aligned16, u32 *__restrict__ tap_bits,
+                                                             int wcols, const __grid_constant__ MorphRuns R)
+{
+    using L = OmLayout<CODE, TR, RUNS>;
+    constexpr int N = L::N, EXT = L::EXT, TILES = L::TILES;
+    extern __shared__ __align__(16) u8 smem[];
+    uint4 *s_sl = reinterpret_cast<uint4 *>(smem);
+    u32 *s_od = reinterpret_cast<u32 *>(smem + L::OFF_OD);
     __shared__ uint2 s_lut8[256];
-    __shared__ u32 s_item[4][TILES][32];
-    expand_lut_init(s_lut8, threadIdx.x, blockDim.x);
-    __syncthreads();
+    __shared__ __align__(8) unsigned long long s_bar[L::NBAR];
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-    // warp unit = (plane, strip, group of 30 word columns), columns fastest: every warp of every CTA has work
-    const long long unit = (long long)blockIdx.x * 4 + wid;
-    if (unit >= n_units) return;                              // whole warps only: the list flush below is warp-wide
-#if ML_ORDER == 3
-    // planes fastest: the 4 warps of a CTA are 4 planes of ONE (strip, column group) -- they load the same label slices / Od words
-    // at about the same time, so three of the four find them in L1
-    const int p = (int)(unit % n_planes);
-    const long long u2 = unit / n_planes;
-    const int wx = (int)(u2 % wcols), strip = (int)(u2 / wcols);
-#else
-    const int wx = (int)(unit % wcols);
-    const long long u2 = unit / wcols;
-#if ML_ORDER == 1
-    const int p = (int)(u2 % n_planes), strip = (int)(u2 / n_planes);       // the planes of a strip run together: they share its label rows
-#else
-    const int strip = (int)(u2 % strips), p = (int)(u2 / strips);
-#endif
-#endif
+    const int wx = (int)(blockIdx.x % (unsigned)wcols);
+    const int u2 = (int)(blockIdx.x / (unsigned)wcols);
+    const int fg = u2 % (nf * groups), strip = u2 / (nf * groups);
+    const int f = fg / groups, grp = fg - f * groups;
     const int ww = (w + 31) >> 5;
-    const int c = wx * LP_COLS - 1 + lane;
-    const bool inimg = c >= 0 && c < ww;
-    const bool owned = inimg && lane >= 1 && lane <= LP_COLS;
-    const int f = p / K, k = p - f * K;
+    const int c = wx * LP_COLS - 1 + lane;                     // the lane's word column = staged column lane + 1
+    const int cs = c - lane - 1;                               // first staged column (c0 - 2)
+    const int lo = max(0, -cs), hi = min(OM_SCOLS, ww - cs);   // staged columns inside the image
     const int y0 = strip * TR, y1 = min(h, y0 + TR);
+    const int ys0 = y0 - N - EXT - 2, rs = y1 - y0 + 2 * (N + EXT + 2);    // staged rows
+    const int yo0 = y0 - N - EXT, ro = y1 - y0 + 2 * (N + EXT);            // Od rows
+    const u32 bar0 = (u32)__cvta_generic_to_shared(s_bar);
+    // ---- 1. staging ----
+    if (threadIdx.x == 0) {
+        for (int j = 0; j < L::NBAR; j++) asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(bar0 + 8u * j));
+        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        const uint4 *src = slices + (size_t)f * plane + cs + lo;
+        const u32 dst0 = (u32)__cvta_generic_to_shared(s_sl + lo), bytes = (u32)(hi - lo) * 16u;
+        for (int j = 0; j * OM_CHUNK < rs; j++) {
+            const int a = max(j * OM_CHUNK, -ys0), b = min(min(rs, (j + 1) * OM_CHUNK), h - ys0);     // rows inside the image
+            asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar0 + 8u * j), "r"(b > a ? (u32)(b - a) * bytes : 0u)
+                         : "memory");
+            for (int r = a; r < b; r++)
+                asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
+                             ::"r"(dst0 + (u32)(r * OM_SCOLS * 16)), "l"(src + (ptrdiff_t)(ys0 + r) * ws), "r"(bytes), "r"(bar0 + 8u * j)
+                             : "memory");
+        }
+    }
+    for (int i = threadIdx.x; i < rs * OM_SCOLS; i += blockDim.x) {
+        const int r = i / OM_SCOLS, col = i - r * OM_SCOLS, y = ys0 + r;
+        if (y < 0 || y >= h || col < lo || col >= hi) s_sl[i] = make_uint4(0u, 0u, 0u, 0u);
+    }
+    expand_lut_init(s_lut8, threadIdx.x, blockDim.x);
+    __syncthreads();                                           // barriers initialised, zeros and LUT written
+    const bool inimg = c >= 0 && c < ww;
+    const u32 colvalid = inimg ? range_mask(32 * c, w) : 0u;
+    // ---- 2. Od of the rows [yo0, yo0 + ro), a segment of rows per warp ----
+    {
+        const int seg = (ro + P - 1) / P;
+        const int ys = yo0 + wid * seg, ye = min(yo0 + ro, ys + seg);
+        if (ys < ye) {
+            const int ra = ys - 2 - ys0, rb = ye + 2 - ys0;    // staged rows the segment reads
+            for (int j = ra / OM_CHUNK; j * OM_CHUNK < rb; j++) om_wait(bar0 + 8u * j);
+            const int ce = lane == 0 ? c - 1 : c + 1;          // lanes 0 / 31: the staged column beyond the lane's
+            const u32 cme = (ce >= 0 && ce < ww) ? range_mask(32 * ce, w) : 0u;
+            const u32 lfix = (c == 0) ? 1u : 0u, lfixe = (ce == 0) ? 1u : 0u;                       // pixel 0 has no left neighbour
+            const u32 rlast = 1u << ((w - 1) & 31);
+            const u32 rfix = (c == ww - 1) ? rlast : 0u, rfixe = (ce == ww - 1) ? rlast : 0u;       // pixel w-1 has no right neighbour
+            const int eidx = lane == 0 ? 0 : OM_SCOLS - 1;
+            u32 sp[4] = {0u, 0u, 0u, 0u}, spe[4] = {0u, 0u, 0u, 0u};
+            u32 dh1 = 0u, dh2 = 0u, dv1 = 0u, hu2 = 0u, hu3 = 0u, dhe1 = 0u, dhe2 = 0u, dve1 = 0u;
+            for (int r = ys - 2; r < ye + 2; r++) {
+                const uint4 *row = s_sl + (r - ys0) * OM_SCOLS;
+                const uint4 v = row[lane + 1], ev = row[eidx];
+                const u32 s[4] = {v.x, v.y, v.z, v.w}, e[4] = {ev.x, ev.y, ev.z, ev.w};
+                const bool rin = r >= 0 && r < h;
+                u32 dl = 0u, dr = 0u, dv = 0u, dle = 0u, dre = 0u, dve = 0u;
+#pragma unroll
+                for (int b = 0; b < 4; b++) {
+                    const u32 m = s[b], x = e[b];
+                    u32 l = __shfl_up_sync(0xffffffffu, m, 1), rr = __shfl_down_sync(0xffffffffu, m, 1);
+                    if (lane == 0) l = x;
+                    if (lane == 31) rr = x;
+                    dl |= m ^ __funnelshift_l(l, m, 1);
+                    dr |= m ^ __funnelshift_r(m, rr, 1);
+                    dv |= m ^ sp[b];
+                    sp[b] = m;
+                    // the extra column: bit 31 of lane 0's (left of m), bit 0 of lane 31's (right of m) are exact
+                    dle |= x ^ (lane == 0 ? (x << 1) : __funnelshift_l(m, x, 1));
+                    dre |= x ^ (lane == 0 ? __funnelshift_r(x, m, 1) : (x >> 1));
+                    dve |= x ^ spe[b];
+                    spe[b] = x;
+                }
+                dl &= ~lfix; dr &= ~rfix; dle &= ~lfixe; dre &= ~rfixe;
+                const u32 dh0 = rin ? (dl | dr) : 0u, dhe0 = rin ? (dle | dre) : 0u;
+                const u32 dv0 = (rin && r > 0) ? dv : 0u, dve0 = (rin && r > 0) ? dve : 0u;
+                const bool yin = r - 1 >= 0 && r - 1 < h;
+                const u32 U = yin ? (~(dh2 | dh1 | dh0 | dv1 | dv0) & colvalid) : 0u;
+                const u32 Ue = yin ? (~(dhe2 | dhe1 | dhe0 | dve1 | dve0) & cme) : 0u;
+                u32 l = __shfl_up_sync(0xffffffffu, U, 1), rr = __shfl_down_sync(0xffffffffu, U, 1);
+                if (lane == 0) l = Ue;
+                if (lane == 31) rr = Ue;
+                const u32 hu1 = U | __funnelshift_l(l, U, 1) | __funnelshift_r(U, rr, 1);
+                const int z = r - 2;
+                if (z >= ys) s_od[(z - yo0) * 32 + lane] = (z >= 0 && z < h) ? ((hu3 | hu2 | hu1) & colvalid) : 0u;
+                hu3 = hu2; hu2 = hu1; dh2 = dh1; dh1 = dh0; dv1 = dv0; dhe2 = dhe1; dhe1 = dhe0; dve1 = dve0;
+            }
+        }
+    }
+    __syncthreads();                                           // Od complete; no CTA-wide barrier after this point
+    const int k = grp * P + wid;
+    if (k >= K) return;                                        // whole warps: the list flush below is warp-wide
+    // ---- 3. the chain of plane p ----
+    const int p = f * K + k;
+    const bool owned = inimg && lane >= 1 && lane <= LP_COLS;
     const int t_first = y0 - N - EXT;
-    // running pointers of the row being fetched (t + 1), the tapped row (t - TAP) and the final row (t - N); they may point
-    // outside the planes while the row is outside [0, h): never dereferenced then
-    const uint4 *sl = slices + (ptrdiff_t)f * (ptrdiff_t)plane + (ptrdiff_t)t_first * ws + c;
-    const u32 *odp = od + (ptrdiff_t)f * (ptrdiff_t)plane + (ptrdiff_t)t_first * ws + c;
+    // running pointers of the tapped row (t - TAP) and the final row (t - N); they may point outside the planes while the row is
+    // outside [0, h): never dereferenced then
     u8 *mrow = masks + (size_t)p * mstride + (ptrdiff_t)(t_first - TAP) * (ptrdiff_t)mpitch;
     u32 *trow = tap_bits + (ptrdiff_t)p * (ptrdiff_t)plane + (ptrdiff_t)(t_first - TAP) * ws + c;
     u32 *frow = out_bits + (ptrdiff_t)p * (ptrdiff_t)plane + (ptrdiff_t)(t_first - N) * ws + c;
     const u32 n0 = (k & 1) ? 0u : 0xffffffffu, n1 = (k & 2) ? 0u : 0xffffffffu, n2 = (k & 4) ? 0u : 0xffffffffu,
               n3 = (k & 8) ? 0u : 0xffffffffu;
-    const u32 colvalid = inimg ? range_mask(32 * c, w) : 0u;
     // pixels 32c-2, 32c-1 (top bits of the left lane's word) and 32c+32, 32c+33 (low bits of the right lane's) inside the image?
     const u32 lv = (c >= 1 && c <= ww) ? 0xC0000000u : 0u;
     const u32 rv = (c + 1 >= 0) ? (range_mask(32 * c + 32, w) & 3u) : 0u;
@@ -520,23 +545,20 @@ __global__ void __launch_bounds__(128, ML_MINB) fk_morph_lab(const uint4 *__rest
     u32 p1[8], p2[8];
 #pragma unroll
     for (int s = 0; s < 8; s++) p1[s] = p2[s] = 0u;
-    // the slice words and Od of the next row are loaded one row ahead and stay RAW in registers until they are needed (combining
-    // them at once would wait for the loads right there)
-    uint4 nsl = make_uint4(0u, 0u, 0u, 0u);
-    u32 nod = 0u;
-    auto fetch = [&](const int t) {
-        nod = 0u;
-        if (t >= 0 && t < h && inimg) { nod = __ldg(odp); nsl = __ldg(sl); }
-        odp += ws; sl += ws;
-    };
+    // the slice words and Od of row t (zeros outside the image), read one row ahead
+    const uint4 *ssl = s_sl + (t_first - ys0) * OM_SCOLS + lane + 1;
+    const u32 *sod = s_od + lane;
+    uint4 nsl;
+    u32 nod;
+    auto fetch = [&]() { nsl = *ssl; nod = *sod; ssl += OM_SCOLS; sod += 32; };
     u32 live1 = 0u, live0 = 0u;
     auto rows = [&](auto rowfix_tag, auto colfix_tag) {
         constexpr bool ROWFIX = decltype(rowfix_tag)::value, COLFIX = decltype(colfix_tag)::value;
-        fetch(t_first);
+        fetch();
         for (int t = t_first; t < y1 + N + EXT; t++) {
             u32 cur = nod & (nsl.x ^ n0) & (nsl.y ^ n1) & (nsl.z ^ n2) & (nsl.w ^ n3);          // open_k = Od & [label == k]
             const bool inside = t >= 0 && t < h;
-            fetch(t + 1);
+            fetch();
             cur = oob_fix32<OP0, ROWFIX, COLFIX>(cur, colvalid, !ROWFIX || inside);
             u32 tap = 0u, fin = 0u;
             MorphChain32<CODE, 0>::template run<TAP, ROWFIX, COLFIX>(cur, p1, p2, t, h, colvalid, tap, fin);
@@ -571,12 +593,15 @@ __global__ void __launch_bounds__(128, ML_MINB) fk_morph_lab(const uint4 *__rest
     else { if (colfix) rows(std::false_type{}, std::true_type{}); else rows(std::false_type{}, std::false_type{}); }
     if (!RUNS) return;
     // ---- run lists of the sparse edge kernel (see fk_morph / fk_edge_runs for the rule and the list layout) ----
+    // a run is kept in the slot of the tile where it is emitted (slot TILES: after the last tile), so that every slot index is a
+    // compile-time constant and the items stay in registers
+    u32 item[TILES + 1];
     const u32 live = owned ? (live1 & live0) : 0u;
-    int n_items = 0, run = 0, run_j0 = 0;
-    u32 lens = 0u;
-    auto emit = [&]() {
-        lens |= (u32)run << (3 * n_items);
-        s_item[wid][n_items++][lane] = ((u32)p << 27) | ((u32)run_j0 << 13) | (u32)c;
+    int run = 0, run_j0 = 0;
+    u32 lens = 0u;                                             // 3 bits per slot: length of its run, 0 = empty
+    auto emit = [&](const int slot) {
+        lens |= (u32)run << (3 * slot);
+        item[slot] = ((u32)p << 27) | ((u32)run_j0 << 13) | (u32)c;
         run = 0;
     };
 #pragma unroll
@@ -585,9 +610,9 @@ __global__ void __launch_bounds__(128, ML_MINB) fk_morph_lab(const uint4 *__rest
         if (ty0 >= y1) break;
         if ((live >> tl) & 1u) {
             if (run == 0) run_j0 = ty0 / ET_R;
-            if (++run == R.maxt) emit();
+            if (++run == R.maxt) emit(tl);
         } else {
-            if (run) emit();
+            if (run) emit(tl);
             if (owned && R.zero_fill) {
                 const int ty1 = min(y1, ty0 + ET_R);
                 for (int y = ty0; y < ty1; y++) {
@@ -598,11 +623,12 @@ __global__ void __launch_bounds__(128, ML_MINB) fk_morph_lab(const uint4 *__rest
             }
         }
     }
-    if (run) emit();
+    if (run) emit(TILES);
 #pragma unroll
     for (int nt = 1; nt <= ET_MAXT; nt++) {
         int mine = 0;
-        for (int i = 0; i < n_items; i++) mine += ((lens >> (3 * i)) & 7u) == (u32)nt;
+#pragma unroll
+        for (int i = 0; i <= TILES; i++) mine += ((lens >> (3 * i)) & 7u) == (u32)nt;
         int x = mine;
 #pragma unroll
         for (int d = 1; d < 32; d <<= 1) {
@@ -615,8 +641,9 @@ __global__ void __launch_bounds__(128, ML_MINB) fk_morph_lab(const uint4 *__rest
         if (lane == 31) base = atomicAdd(R.run_counts + nt - 1, total);
         base = __shfl_sync(0xffffffffu, base, 31);
         int pos = base + x - mine;
-        for (int i = 0; i < n_items; i++)
-            if (((lens >> (3 * i)) & 7u) == (u32)nt) R.run_items[R.off.v[nt - 1] + pos++] = s_item[wid][i][lane];
+#pragma unroll
+        for (int i = 0; i <= TILES; i++)
+            if (((lens >> (3 * i)) & 7u) == (u32)nt) R.run_items[R.off.v[nt - 1] + pos++] = item[i];
     }
 }
 
@@ -655,38 +682,65 @@ constexpr u32 CODE_L_O = mk_code(ST_DR, ST_ER, ST_EC, ST_DC);
 constexpr u32 CODE_L_C = mk_code(ST_DR, ST_ER, ST_DC, ST_EC);
 constexpr u32 CODE_L_OC = mk_code(ST_DR, ST_ER, ST_EC, ST_DC, ST_DC, ST_EC);
 
-static cudaError_t launch_morph_lab(int kind /* -1: masks only */, const uint4 *slices, const u32 *od, u32 *m2, const BitGeom &g, int K, int KT,
-                                    u8 *masks, size_t mstride, size_t mpitch, u32 *tap_bits, const MorphRuns &R, cudaStream_t st)
+// the dynamic shared memory of fk_open_morph may exceed the 48 KB default: raise the limit once per device and instance
+template <u32 CODE, int TR, bool RUNS>
+static cudaError_t open_morph_smem_attr()
 {
+    static unsigned done = 0;                                  // bit d: set on device d
+    int dev = 0;
+    if (cudaGetDevice(&dev) != cudaSuccess) return cudaGetLastError();
+    if (dev < 32 && ((done >> dev) & 1u)) return cudaSuccess;
+    const cudaError_t e = cudaFuncSetAttribute(fk_open_morph<CODE, 2, TR, RUNS>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                               (int)OmLayout<CODE, TR, RUNS>::bytes());
+    if (e == cudaSuccess && dev < 32) done |= 1u << dev;
+    return e;
+}
+
+static cudaError_t launch_open_morph(int kind /* -1: masks only */, const uint4 *slices, u32 *m2, const BitGeom &g, int K, int nf,
+                                     u8 *masks, size_t mstride, size_t mpitch, u32 *tap_bits, const MorphRuns &R, cudaStream_t st)
+{
+    const int KT = nf * K;
     const int wcols = (g.ww + LP_COLS - 1) / LP_COLS;
     const int al = plane_align(masks, mstride, mpitch);
-    // Strip height.  A warp walks its strip row by row (+ ~20 rows of halo and pipeline), and the kernel is latency-bound: its time is
-    // about  waves x (rows + 20),  waves = ceil(strip-warps / resident warps).  Short strips for small grids (one wave: the shortest
-    // walk wins), tall ones once there are several waves, and 56 rows where that lands the grid on a whole number of waves
-    // (4096^2: 2960 resident warps = the 5 x 74 x 8 strip-warps of K = 8, half those of K = 16).
+    // planes of one frame per CTA: the fewest groups of at most OM_PMAX planes, as even as possible
+    const int groups = (K + OM_PMAX - 1) / OM_PMAX, P = (K + groups - 1) / groups;
+    // Strip height.  A warp walks its strip row by row (+ ~20 rows of halo and pipeline): the kernel's time is about
+    // waves x (rows + 20),  waves = ceil(strip-warps / resident warps).  Short strips for small grids (one wave: the shortest walk
+    // wins), tall ones once there are several waves, and 56 rows where that lands the grid on a whole number of waves.
 #ifdef ML_TR
     const int tr = ML_TR;
 #else
-    static int resident = 0;
-    if (resident == 0) {
-        int per_sm = 0, dev = 0, sms = 0;
-        if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, fk_morph_lab<CODE_L_OC, 2, 64, true>, 128, 0) != cudaSuccess || per_sm < 1) per_sm = 4;
+    // resident warps per TR candidate (shared memory grows with TR), per CTA size
+    static int resident[OM_PMAX + 1][3] = {};
+    const int cands[3] = {32, 56, 64};
+    if (resident[P][0] == 0) {
+        int dev = 0, sms = 0;
         if (cudaGetDevice(&dev) != cudaSuccess || cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess || sms < 1) sms = 148;
+        auto occ = [&](auto kern, cudaError_t attr, size_t smem) {
+            int per_sm = 0;
+            if (attr != cudaSuccess || cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, 32 * P, smem) != cudaSuccess || per_sm < 1) per_sm = 1;
+            return per_sm * P * sms;
+        };
+        resident[P][0] = occ(fk_open_morph<CODE_L_OC, 2, 32, true>, open_morph_smem_attr<CODE_L_OC, 32, true>(), OmLayout<CODE_L_OC, 32, true>::bytes());
+        resident[P][1] = occ(fk_open_morph<CODE_L_OC, 2, 56, true>, open_morph_smem_attr<CODE_L_OC, 56, true>(), OmLayout<CODE_L_OC, 56, true>::bytes());
+        resident[P][2] = occ(fk_open_morph<CODE_L_OC, 2, 64, true>, open_morph_smem_attr<CODE_L_OC, 64, true>(), OmLayout<CODE_L_OC, 64, true>::bytes());
         cudaGetLastError();
-        resident = per_sm * 4 * sms;
     }
     int tr = 32;
     long long best = -1;
-    for (int cand : {32, 56, 64}) {
+    for (int i = 0; i < 3; i++) {
+        const int cand = cands[i], res = resident[P][i];
         const long long units = (long long)wcols * ((g.h + cand - 1) / cand) * KT;
-        const long long cost = ((units + resident - 1) / resident) * (cand + 20);
+        const long long cost = ((units + res - 1) / res) * (cand + 20);
         if (best < 0 || cost <= best) { best = cost; tr = cand; }
     }
 #endif
     const int strips = (g.h + tr - 1) / tr;
-    const long long n_units = (long long)wcols * strips * KT;
-    dim3 b(128), grid((unsigned)((n_units + 3) / 4));
-#define LL2(CODE, TRV, RUNS) fk_morph_lab<CODE, 2, TRV, RUNS><<<grid, b, 0, st>>>(slices, od, m2, g.ws, g.plane, g.h, g.w, K, masks, mstride, mpitch, al, tap_bits, wcols, strips, KT, n_units, R)
+    const dim3 grid((unsigned)((long long)wcols * groups * nf * strips)), b(32 * P);
+    cudaError_t e = cudaSuccess;
+#define LL2(CODE, TRV, RUNS) do { if ((e = open_morph_smem_attr<CODE, TRV, RUNS>()) != cudaSuccess) return e; \
+        fk_open_morph<CODE, 2, TRV, RUNS><<<grid, b, OmLayout<CODE, TRV, RUNS>::bytes(), st>>>(slices, m2, g.ws, g.plane, g.h, g.w, K, P, groups, nf, \
+                                                 masks, mstride, mpitch, al, tap_bits, wcols, R); } while (0)
 #ifdef ML_TR
 #define LL(CODE, RUNS) LL2(CODE, ML_TR, RUNS)
 #else
@@ -722,14 +776,14 @@ static int label_pipeline(omni_ctx *ctx, const u8 *d_bgr, int nf, size_t frame_s
     const BitGeom g = make_geom(h, w);
     if ((long long)nf * h * ((w + 255) >> 8) >= (1ll << 30)) return OMNI_ERR_UNSUPPORTED;
     OMNI_CUDA(fast_tables());
-    // ---- workspace (slot 4): [label slices 4 nf | Od nf | M2 KT | S KT | C KT | mask bits KT]; S and C laid out as edge_pass_begin expects
+    // ---- workspace (slot 4): [label slices 4 nf | M2 KT | S KT | C KT | mask bits KT]; S and C laid out as edge_pass_begin expects
     const size_t pbytes = g.plane * sizeof(u32);
     auto al = [](size_t v) { return (v + 255) & ~(size_t)255; };
-    const size_t o_sl = 0, o_od = al(o_sl + pbytes * 4 * nf), o_m2 = al(o_od + pbytes * nf), o_s = al(o_m2 + pbytes * KT),
+    const size_t o_sl = 0, o_m2 = al(o_sl + pbytes * 4 * nf), o_s = al(o_m2 + pbytes * KT),
                  o_c = o_s + al(pbytes * KT), o_mb = al(o_c + pbytes * KT), bits_total = al(o_mb + (want_mask_bits ? pbytes * KT : 0));
     SP_TRY(omni_ws_reserve(ctx, 4, bits_total));           // (label_ws_bytes() below states the same sizes for omni_workspace_bytes)
     u8 *b4 = (u8 *)ctx->ws[4];
-    u32 *slices = (u32 *)(b4 + o_sl), *od = (u32 *)(b4 + o_od), *M2 = (u32 *)(b4 + o_m2), *sbits = (u32 *)(b4 + o_s), *cbits = (u32 *)(b4 + o_c);
+    u32 *slices = (u32 *)(b4 + o_sl), *M2 = (u32 *)(b4 + o_m2), *sbits = (u32 *)(b4 + o_s), *cbits = (u32 *)(b4 + o_c);
     u32 *mbits = want_mask_bits ? (u32 *)(b4 + o_mb) : nullptr;
     if (out) { out->slices = slices; out->mask_bits = mbits; out->edge_bits = prm ? sbits : nullptr; out->cand_bits = prm ? cbits : nullptr; }
     // the zeros of the dead edge tiles: byte planes -> they ride on the assignment kernel (ZeroJob; strided planes: side stream);
@@ -766,19 +820,10 @@ static int label_pipeline(omni_ctx *ctx, const u8 *d_bgr, int nf, size_t frame_s
                                                                                  lpitch, slices, g.ws, nf, frame_stride, Z);
         OMNI_CUDA(cudaGetLastError());
     }
-    // ---- 2. label-domain open: Od ----
-    {
-        const int wcols = (g.ww + LP_COLS - 1) / LP_COLS, strips = (h + LO_ROWS - 1) / LO_ROWS;
-        const long long warps = (long long)nf * strips * wcols;
-        KScope ks(ctx, "label_open", st);
-        fk_label_open<<<(unsigned)((warps + LO_WARPS - 1) / LO_WARPS), LO_WARPS * 32, 0, st>>>((const uint4 *)slices, g.ws, g.plane, h, w, nf, od, strips,
-                                                                                              wcols);
-        OMNI_CUDA(cudaGetLastError());
-    }
-    // ---- 3. the rest of the morphology chain per plane, run lists for the edge kernel ----
-    OMNI_LAUNCH(ctx, st, "morph_bits", launch_morph_lab(kind, (const uint4 *)slices, od, M2, g, K, KT, d_masks, m_plane, mpitch, mbits, R, st));
+    // ---- 2. label-domain open and the rest of the morphology chain per plane, run lists for the edge kernel ----
+    OMNI_LAUNCH(ctx, st, "morph_bits", launch_open_morph(kind, (const uint4 *)slices, M2, g, K, nf, d_masks, m_plane, mpitch, mbits, R, st));
     if (!prm) return OMNI_OK;
-    // ---- 4. edges on the live tile runs, hysteresis ----
+    // ---- 3. edges on the live tile runs, hysteresis ----
     if (ctx->edge_join) {                               // the side stream has cleared the output planes
         OMNI_CUDA(cudaStreamWaitEvent(st, ctx->edge_join, 0));
         ctx->edge_join = nullptr;
@@ -799,8 +844,7 @@ void label_ws_bytes(int h, int w, int K, int nf, size_t out[OMNI_WS_SLOTS])
     const int KT = nf * K;
     const size_t pbytes = g.plane * sizeof(u32);
     auto al = [](size_t v) { return (v + 255) & ~(size_t)255; };
-    const size_t o_od = al(pbytes * 4 * nf), o_m2 = al(o_od + pbytes * nf), o_s = al(o_m2 + pbytes * KT), o_c = o_s + al(pbytes * KT),
-                 o_mb = al(o_c + pbytes * KT);
+    const size_t o_m2 = al(pbytes * 4 * nf), o_s = al(o_m2 + pbytes * KT), o_c = o_s + al(pbytes * KT), o_mb = al(o_c + pbytes * KT);
     unsigned off[ET_MAXT];
     out[4] = std::max(out[4], al(o_mb + pbytes * KT));
     out[5] = std::max(out[5], WS5_BYTES + WS5_LABEL_BYTES);

@@ -15,7 +15,7 @@ KEYS = ["gpu__time_duration.sum", "dram__bytes_read.sum", "dram__bytes_write.sum
         "launch__block_size", "sm__throughput.avg.pct_of_peak_sustained_elapsed",
         "gpu__dram_throughput.avg.pct_of_peak_sustained_elapsed", "l1tex__t_sector_hit_rate.pct", "lts__t_sector_hit_rate.pct"]
 BENCH_NAME = {"fk_assign_rgbcell": "assign_bits", "fk_assign_bits": "assign_bits", "fk_assign_slices": "assign_bits", "fk_morph": "morph_bits",
-              "fk_morph_lab": "morph_bits", "fk_label_open": "label_open", "fk_build_tables3": "build_tables",
+              "fk_morph_lab": "morph_bits", "fk_label_open": "label_open", "fk_open_morph": "morph_bits", "fk_build_tables3": "build_tables",
               "fk_edges3_simd": "edges3_bits", "fk_hysteresis": "hysteresis_bits", "fk_edge_runs": "edge_runs", "fk_thin": "thin_zhangsuen"}
 UNIT = {"Mbyte": 1e6, "Kbyte": 1e3, "Gbyte": 1e9, "byte": 1.0}
 
