@@ -38,7 +38,7 @@ extern "C" {
 #define OMNI_ABI_VERSION 1
 #define OMNI_MAX_K 32            /* colour layers per image (labels are u8; reference configs use 4..16) */
 #define OMNI_MAX_BLUR_K 31       /* largest edge_kernel_size with a built-in 8.8 weight table */
-#define OMNI_MAX_MORPH_K 7       /* largest edge_morph_kernel */
+#define OMNI_MAX_MORPH_K 255     /* largest edge_morph_kernel (element offsets are int8: +-127) */
 
 #define OMNI_OK 0
 #define OMNI_ERR_ARG (-1)
@@ -50,9 +50,9 @@ typedef struct omni_ctx omni_ctx;
 
 /* 03_edge_detect.py:23-34 knobs, as read from config.json (config.py:31-36). */
 typedef struct omni_edge_params {
-    int32_t morph_k;      /* edge_morph_kernel: ELLIPSE structuring element size, >= 1            */
-    int32_t open_iters;   /* edge_morph_open_iters  (<= 0: skip)                                  */
-    int32_t close_iters;  /* edge_morph_close_iters (<= 0: skip)                                  */
+    int32_t morph_k;      /* edge_morph_kernel: ELLIPSE structuring element size, 1..OMNI_MAX_MORPH_K */
+    int32_t open_iters;   /* edge_morph_open_iters  (<= 0: skip; any positive count)              */
+    int32_t close_iters;  /* edge_morph_close_iters (<= 0: skip; any positive count)              */
     int32_t ksize;        /* edge_kernel_size after _ensure_odd (03:9-11): odd, >= 3              */
     double low, high;     /* edge_low_threshold / edge_high_threshold exactly as given to Canny   */
 } omni_edge_params;

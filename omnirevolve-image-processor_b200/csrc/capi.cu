@@ -233,12 +233,11 @@ int omni_ws_reserve(omni_ctx *ctx, int slot, size_t bytes)
 }
 
 // ---- host-side parameter preparation --------------------------------------------------------------
-// cv2.getStructuringElement(MORPH_RECT | MORPH_ELLIPSE, (k,k)) as an offset list (SURVEY A.0).
+// cv2.getStructuringElement(MORPH_RECT | MORPH_ELLIPSE, (k,k)) as one span per row (SURVEY A.0).
 void omni_build_se(int shape_ellipse, int k, MorphSE *se)
 {
     int r = k / 2, c = k / 2, a = k / 2;
     double inv_r2 = r ? 1.0 / ((double)r * r) : 0.0;
-    se->n = 0;
     se->k = k;
     for (int i = 0; i < k; i++) {
         int j1 = 0, j2 = 0;
@@ -251,7 +250,8 @@ void omni_build_se(int shape_ellipse, int k, MorphSE *se)
                 j2 = c + dx + 1 < k ? c + dx + 1 : k;
             }
         }
-        for (int j = j1; j < j2; j++) { se->dy[se->n] = (int8_t)(i - a); se->dx[se->n] = (int8_t)(j - a); se->n++; }
+        se->x0[i] = (int8_t)(j1 - a);                  // |j - a| <= 127 for k <= 255
+        se->x1[i] = (int8_t)(j2 - 1 - a);
     }
 }
 
@@ -502,7 +502,6 @@ static int check_edge_params(const omni_edge_params *p, BlurParams *bp, int *low
 {
     OMNI_REQUIRE(p != nullptr, "edge params NULL");
     OMNI_REQUIRE(p->morph_k >= 1 && p->morph_k <= OMNI_MAX_MORPH_K, "edge_morph_kernel=%d outside [1,%d]", p->morph_k, OMNI_MAX_MORPH_K);
-    OMNI_REQUIRE(p->open_iters <= 32 && p->close_iters <= 32, "edge morph iterations too large");
     if (omni_gauss_weights(p->ksize, bp)) {
         omni_set_error("edge_kernel_size=%d: need an odd size in [3,%d] (apply _ensure_odd first)", p->ksize, OMNI_MAX_BLUR_K);
         return OMNI_ERR_UNSUPPORTED;
@@ -545,17 +544,15 @@ static int generic_edges(omni_ctx *ctx, const uint8_t *d_masks, int K, int h, in
     u8 *A = (u8 *)ctx->ws[0], *B = (u8 *)ctx->ws[1];
     MorphSE se;
     omni_build_se(1, prm->morph_k, &se);
-    int oi = prm->open_iters > 0 ? prm->open_iters : 0, ci = prm->close_iters > 0 ? prm->close_iters : 0;
+    long long oi = prm->open_iters > 0 ? prm->open_iters : 0, ci = prm->close_iters > 0 ? prm->close_iters : 0;
     if (skip_morph) oi = ci = 0;
-    int seq_n = 0, seq[4 * 64];
-    for (int i = 0; i < oi; i++) seq[seq_n++] = 0;
-    for (int i = 0; i < oi; i++) seq[seq_n++] = 1;
-    for (int i = 0; i < ci; i++) seq[seq_n++] = 1;
-    for (int i = 0; i < ci; i++) seq[seq_n++] = 0;
+    // OPEN = erode^oi dilate^oi ; CLOSE = dilate^ci erode^ci (cv2 loops the iterations of a non-rectangular element)
+    const long long n_steps = 2 * (oi + ci);
     const u8 *cur = d_masks; size_t cplane = m_plane, cpitch = mpitch;
-    for (int i = 0; i < seq_n; i++) {
+    for (long long i = 0; i < n_steps; i++) {
+        const int dilate = (i >= oi && i < 2 * oi + ci) ? 1 : 0;
         u8 *dst = (cur == A) ? B : A;
-        OMNI_LAUNCH(ctx, st, "morph", g_morph(cur, cplane, cpitch, dst, wplane, wp, K, h, w, se, seq[i], st));
+        OMNI_LAUNCH(ctx, st, "morph", g_morph(cur, cplane, cpitch, dst, wplane, wp, K, h, w, se, dilate, st));
         cur = dst; cplane = wplane; cpitch = wp;
     }
     u8 *bl = (cur == A) ? B : A;
@@ -565,7 +562,9 @@ static int generic_edges(omni_ctx *ctx, const uint8_t *d_masks, int K, int h, in
 }
 
 // masks (byte planes) -> edges with the best available kernels:
-//   fast bit-plane path (edge_kernel_size 3) > fast bit morphology + generic blur/Canny (other sizes) > generic
+//   fast bit-plane path (edge_kernel_size 3 / 5 / 7) > fast bit morphology + generic blur/Canny (other sizes) > generic.
+//   The bit morphology is fk_morph for morph_k 1 and 3 with at most one open / close, the ELLIPSE kernel of morph_ellipse.cu
+//   for every other size and count; masks that are not strictly {0,255} take the generic kernels.
 static int edges_dispatch(omni_ctx *ctx, const uint8_t *d_masks, int K, int h, int w, size_t m_plane, size_t mpitch,
                           const omni_edge_params *prm, const BlurParams &bp, int low, int high,
                           uint8_t *d_edges, size_t e_plane, size_t epitch, cudaStream_t st)

@@ -170,6 +170,10 @@ int run_hysteresis_wl(omni_ctx *ctx, u32 *ebits, const u32 *cbits, const BitGeom
 int edge_pass_begin(omni_ctx *ctx, const BitGeom &g, int K, u32 *sbits, u32 *cbits, u8 *d_edges, size_t e_plane, size_t epitch,
                     cudaStream_t st, MorphRuns *R, bool *sparse, bool side_fill, ZeroJob *zjob = nullptr);
 int morph03_kind(const omni_edge_params *p);
+// stage-03 open/close with the ELLIPSE(morph_k) element for any size and count (morph_ellipse.cu): planes in a, b is scratch;
+// *result = whichever of the two holds the end
+int ellipse_morph_bits(omni_ctx *ctx, const omni_edge_params *prm, const BitGeom &g, int K, u32 *a, u32 *b, const u32 **result,
+                       cudaStream_t st);
 
 // shared-memory layout of the table-driven assignment kernels (fk_assign_rgbcell, fk_assign_slices)
 #define RA_THREADS 1024

@@ -1440,14 +1440,18 @@ int morph03_kind(const omni_edge_params *p)
     return oi | (ci << 1);
 }
 
+// stage-03 morphology on bit-planes: fk_morph's chains (morph03_kind >= 0) or the ELLIPSE kernel of morph_ellipse.cu (every other
+// element size and iteration count)
+static bool morph03_bits_ok(const omni_edge_params *p) { return morph03_kind(p) >= 0 || (p->morph_k >= 2 && p->morph_k <= OMNI_MAX_MORPH_K); }
+
 bool fast_edges_supported(const omni_edge_params *prm)
 {
-    return morph03_kind(prm) >= 0 && (prm->ksize == 3 || prm->ksize == 5 || prm->ksize == 7);
+    return morph03_bits_ok(prm) && (prm->ksize == 3 || prm->ksize == 5 || prm->ksize == 7);
 }
 
 bool fast_fused_supported(const omni_edge_params *prm) { return morph03_kind(prm) >= 0 && prm->ksize == 3; }
 
-bool fast_morph03_supported(const omni_edge_params *prm) { return morph03_kind(prm) >= 0; }
+bool fast_morph03_supported(const omni_edge_params *prm) { return morph03_bits_ok(prm); }
 
 int fast_morph03_bytes(omni_ctx *ctx, const u8 *d_masks, int K, int h, int w, size_t m_plane, size_t mpitch,
                        const omni_edge_params *prm, u8 *d_out, size_t o_plane, size_t opitch, cudaStream_t st)
@@ -1472,6 +1476,8 @@ int fast_morph03_bytes(omni_ctx *ctx, const u8 *d_masks, int K, int h, int w, si
     if (kind > 0) {
         OMNI_LAUNCH(ctx, st, "morph_bits", launch_morph(false, kind, bpp[0], bpp[1], g, K, nullptr, 0, 0, st));
         m2 = bpp[1];
+    } else if (kind < 0) {
+        FK_TRY(ellipse_morph_bits(ctx, prm, g, K, bpp[0], bpp[1], &m2, st));
     }
     int al = plane_align(d_out, o_plane, opitch);
     KScope ks(ctx, "expand_bits", st);
@@ -1612,13 +1618,15 @@ int fast_edges(omni_ctx *ctx, const u8 *d_masks, int K, int h, int w, size_t m_p
     bool sparse = false;
     const int ks = prm->ksize;
     FK_TRY(edge_pass_begin(ctx, g, K, bpp[2], bpp[3], d_edges, e_plane, epitch, st, &R, &sparse, false));
-    // a tile is dead when the tile grown by the radius of blur + Sobel is uniform; only the morphology kernel classifies with a
-    // growth other than 2, so blur 5 / 7 without stage-03 morphology takes the dense edge kernel
+    // a tile is dead when the tile grown by the radius of blur + Sobel is uniform; only fk_morph classifies with a growth other
+    // than 2, so blur 5 / 7 without stage-03 morphology, or after the ELLIPSE kernel (kind < 0), takes the dense edge kernel
     R.grow = ks == 3 ? 2 : ks == 5 ? 3 : 4;
     if (ks != 3 && kind <= 0) sparse = false;
     if (kind > 0) {
         OMNI_LAUNCH(ctx, st, "morph_bits", launch_morph(false, kind, bpp[0], bpp[1], g, K, nullptr, 0, 0, st, 0, -1, sparse ? &R : nullptr));
         m2 = bpp[1];
+    } else if (kind < 0) {                               // other ELLIPSE sizes / counts: the run lists come from edge_runs
+        FK_TRY(ellipse_morph_bits(ctx, prm, g, K, bpp[0], bpp[1], &m2, st));
     }
     const u8 *blur = nullptr;
     size_t bp_pitch = 0, bp_plane = 0;

@@ -189,11 +189,15 @@ __global__ void k_morph(const u8 *__restrict__ src, size_t s_plane, size_t spitc
     if (x >= w || y >= h) return;
     const u8 *s = src + blockIdx.z * s_plane;
     int v = is_dilate ? 0 : 255;
-    for (int i = 0; i < se.n; i++) {
-        int yy = y + se.dy[i], xx = x + se.dx[i];
-        if (yy < 0 || yy >= h || xx < 0 || xx >= w) continue;
-        int p = s[(size_t)yy * spitch + xx];
-        v = is_dilate ? max(v, p) : min(v, p);
+    for (int i = 0; i < se.k; i++) {                       // row i of the element: dy = i - k/2, dx in [x0[i], x1[i]]
+        const int yy = y + i - se.k / 2;
+        if (yy < 0 || yy >= h) continue;
+        const u8 *row = s + (size_t)yy * spitch;
+        const int xa = max(0, x + se.x0[i]), xb = min(w - 1, x + se.x1[i]);
+        for (int xx = xa; xx <= xb; xx++) {
+            const int p = row[xx];
+            v = is_dilate ? max(v, p) : min(v, p);
+        }
     }
     dst[blockIdx.z * d_plane + (size_t)y * dpitch + x] = (u8)v;
 }

@@ -41,10 +41,9 @@ struct BlurParams {
     u16 w[OMNI_MAX_BLUR_K];
     int k;
 };
-struct MorphSE {               // structuring element as offsets, anchor k/2 (un-reflected, SURVEY A.0)
-    int8_t dy[OMNI_MAX_MORPH_K * OMNI_MAX_MORPH_K];
-    int8_t dx[OMNI_MAX_MORPH_K * OMNI_MAX_MORPH_K];
-    int n;
+struct MorphSE {               // structuring element as row spans, anchor (k/2, k/2), un-reflected (SURVEY A.0):
+    int8_t x0[OMNI_MAX_MORPH_K];   // row i (dy = i - k/2) covers dx in [x0[i], x1[i]]; every row of RECT / ELLIPSE is non-empty
+    int8_t x1[OMNI_MAX_MORPH_K];
     int k;
 };
 struct ResizeTabDev {          // fractional INTER_AREA tables on the device (per axis: ofs[D+1], si[], alpha[])

@@ -11,7 +11,7 @@ LIB_PATH = os.environ.get("OMNI_B200_LIB") or os.path.join(os.path.dirname(_HERE
 
 OMNI_MAX_K = 32
 OMNI_MAX_BLUR_K = 31
-OMNI_MAX_MORPH_K = 7
+OMNI_MAX_MORPH_K = 255
 ERR_UNSUPPORTED = -3
 BITS_LSB_FIRST = 0      # pixel x = bit (x & 7) of byte x >> 3
 BITS_MSB_FIRST = 1      # pixel x = bit 7 - (x & 7): the scanline of a 1-bit PNG, numpy.packbits default
