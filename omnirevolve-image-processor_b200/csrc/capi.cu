@@ -220,6 +220,9 @@ extern "C" int omni_profile_summary(omni_ctx *ctx, char *buf, size_t buflen)
 int omni_ws_reserve(omni_ctx *ctx, int slot, size_t bytes)
 {
     if (ctx->ws_bytes[slot] >= bytes) return OMNI_OK;
+    // the candidate tables of both cache generations live in slot 5: a new allocation holds none of them (it may even come back
+    // at the old address, so no pointer comparison can tell)
+    if (slot == 5) ctx->cells_valid = ctx->cells3_valid = 0;
     if (ctx->ws[slot]) { OMNI_CUDA(cudaFree(ctx->ws[slot])); ctx->ws[slot] = nullptr; ctx->ws_bytes[slot] = 0; }
     size_t want = bytes + bytes / 8;
     cudaError_t e = cudaMalloc(&ctx->ws[slot], want);
@@ -694,7 +697,7 @@ static int packed_device(omni_ctx *ctx, const u8 *d_bgr, int nf, size_t frame_st
         rc = label_color_edge_packed(ctx, d_bgr, nf, frame_stride, h, w, pitch, P, prm, low, high, d_mb, mb_plane, mb_pitch, d_eb, eb_plane,
                                      eb_pitch, bit_order == OMNI_BITS_MSB_FIRST, dc, st);
     if (rc != OMNI_ERR_UNSUPPORTED) return rc;
-    // any other family: byte planes in workspace slot 3's tail, then packed
+    // any other family: byte planes in workspace slot 2, then packed
     const size_t bp_pitch = ((size_t)w + 15) & ~(size_t)15, bplane = bp_pitch * h, lp = bp_pitch;
     const int KT = nf * K;
     OMNI_TRY(omni_ws_reserve(ctx, 2, lp * h + 2 * bplane * KT));

@@ -658,12 +658,12 @@ static int label_tables(omni_ctx *ctx, const AssignParams &P, u32 **cells, u8 **
     SP_TRY(omni_ws_reserve(ctx, 5, WS5_BYTES + WS5_LABEL_BYTES));
     *cells = (u32 *)((u8 *)ctx->ws[5] + WS5_BYTES);
     *rtab = (u8 *)(*cells + CELL_COUNT);
-    if ((ctx->table_cache || ctx->tables_hold) && ctx->cells3_valid && ctx->cells3_ws == ctx->ws[5] && ctx->cells3_stream == (void *)st && ctx->cells3_K == P.K &&
+    if ((ctx->table_cache || ctx->tables_hold) && ctx->cells3_valid && ctx->cells3_stream == (void *)st && ctx->cells3_K == P.K &&
         memcmp(ctx->cells3_c, P.c, sizeof(float) * 3 * P.K) == 0 && memcmp(ctx->cells3_lut, P.lut, P.K) == 0)
         return OMNI_OK;
     memcpy(ctx->cells3_c, P.c, sizeof(float) * 3 * P.K);
     memcpy(ctx->cells3_lut, P.lut, P.K);
-    ctx->cells3_K = P.K; ctx->cells3_stream = (void *)st; ctx->cells3_valid = 1; ctx->cells3_ws = ctx->ws[5];
+    ctx->cells3_K = P.K; ctx->cells3_stream = (void *)st; ctx->cells3_valid = 1;
     if (!ctx->d_rgb_boxes3) {                          // centre-independent: once per context
         SP_TRY(fast_rgb_boxes(ctx, st));
         OMNI_CUDA(cudaMalloc(&ctx->d_rgb_boxes3, (size_t)RC_COUNT * sizeof(uint2)));

@@ -90,14 +90,15 @@ struct omni_ctx {
     cudaEvent_t pipe_ev[24] = {};          // 8 H2D bands, 8 morph bands, 4 pipeline joins, 2 zero-fill fork/join
     cudaEvent_t edge_join = nullptr;        // pending join of the zero-fill side stream (edge_pass_begin -> edges_from_bits)
     int occ_assign_lab = 0, occ_assign_pal = 0, occ_assign_rgb = 0, occ_assign_i16 = 0;   // resident CTAs per SM of the persistent assignment kernels
-    // centres the candidate-cell table in ws[5] was built for (fast colour assignment)
+    // centres the candidate-cell table in ws[5] was built for (fast colour assignment); cleared by omni_ws_reserve when it
+    // reallocates ws[5] and by omni_set_table_cache(0)
     int cells_valid = 0, cells_K = 0;
     void *cells_stream = nullptr;
     float cells_c[OMNI_MAX_K * 3];
     u8 cells_lut[OMNI_MAX_K] = {};
-    // the same for the tables of the sparse generation (label_pipe.cu; tail of ws[5])
+    // the same for the tables of the sparse generation (label_pipe.cu; tail of ws[5]), cleared in the same two places
     int cells3_valid = 0, cells3_K = 0;
-    void *cells3_stream = nullptr, *cells3_ws = nullptr;
+    void *cells3_stream = nullptr;
     float cells3_c[OMNI_MAX_K * 3];
     u8 cells3_lut[OMNI_MAX_K] = {};
     u8 *d_rgb_boxes3 = nullptr;                // d_rgb_boxes in the cell order of fk_assign_slices
