@@ -149,6 +149,17 @@ int omni_swatch_masks(omni_ctx *ctx, const uint8_t *d_bgr, int h, int w, size_t 
  * within 2 % of cv2.kmeans' on the same sample (tests/test_gpu_kmeans.py).  Synchronises the stream (centres go to the host). */
 int omni_kmeans_lab(omni_ctx *ctx, const uint8_t *d_bgr, int h, int w, size_t pitch, const int32_t *h_sample_idx, int n_samples,
                     int K, int attempts, int max_iter, double eps, uint64_t seed, float *h_centers, double *h_compactness, void *stream);
+/* The same for n_frames equally sized frames, frame f at d_bgr + f*frame_stride, each clustered on its own with the same sample
+ * indices (the reference's subsample depends only on the pixel count; NULL = every pixel) and criteria.  h_centers: [n_frames][K][3];
+ * h_compactness: [n_frames] or NULL.  Frame f's centres and compactness are bit-identical to omni_kmeans_lab on that frame: every
+ * (frame, attempt) pair is an independent run of the same kernels, and the most compact attempt wins (ties: the lowest attempt).
+ * All runs of a chunk of frames share each launch.  A chunk holds as many frames as fit in 256 MiB of workspace (per frame:
+ * 4 * n_samples * (attempts + 1) bytes plus ~1.4 KB per attempt), at least one; the workspace is slot 6 of the ctx, which
+ * omni_workspace_bytes / omni_ctx_reserve do not cover (k-means is not part of the fused calls' geometry).
+ * Synchronises the stream. */
+int omni_kmeans_lab_batch(omni_ctx *ctx, const uint8_t *d_bgr, int n_frames, size_t frame_stride, int h, int w, size_t pitch,
+                          const int32_t *h_sample_idx, int n_samples, int K, int attempts, int max_iter, double eps,
+                          uint64_t seed, float *h_centers, double *h_compactness, void *stream);
 
 /* ---- stage 03: 03_edge_detect.py:23-34 per layer ------------------------------------------- */
 /* K independent planes: ELLIPSE(morph_k) open/close -> GaussianBlur(ksize, sigma 0) -> Canny(low,
@@ -212,6 +223,22 @@ int omni_host_color_edge_packed(omni_ctx *ctx, const uint8_t *h_bgr, int n_frame
                                 uint8_t *h_mask_bits, size_t mb_plane_stride, size_t mb_pitch,
                                 uint8_t *h_edge_bits, size_t eb_plane_stride, size_t eb_pitch, int bit_order,
                                 int64_t *h_counts);
+/* Per-frame centres: as omni_color_edge_packed / omni_host_color_edge_packed, except that frame f is assigned with its own centres
+ * h_centers + f*K*3 ([n_frames][K][3]) and LUT h_luts + f*K ([n_frames][K], or NULL: identity) -- photos or video shots with
+ * palettes of their own (e.g. from omni_kmeans_lab_batch), still grouped n_frames * K <= OMNI_MAX_K planes per device pass.
+ * Frame f's planes and counts are those of omni_color_edge_packed with that frame's centres and LUT.  Every frame's LUT is checked
+ * before any work.  In the default family each frame of a group gets its own candidate-table build and assignment launch, and the
+ * group shares the morphology / edge / hysteresis launches. */
+int omni_color_edge_packed_frames(omni_ctx *ctx, const uint8_t *d_bgr, int n_frames, size_t frame_stride, int h, int w, size_t pitch,
+                                  const float *h_centers, int K, const uint8_t *h_luts, const omni_edge_params *prm,
+                                  uint8_t *d_mask_bits, size_t mb_plane_stride, size_t mb_pitch,
+                                  uint8_t *d_edge_bits, size_t eb_plane_stride, size_t eb_pitch, int bit_order,
+                                  int64_t *h_counts, void *stream);
+int omni_host_color_edge_packed_frames(omni_ctx *ctx, const uint8_t *h_bgr, int n_frames, size_t frame_stride, int h, int w, size_t pitch,
+                                       const float *h_centers, int K, const uint8_t *h_luts, const omni_edge_params *prm,
+                                       uint8_t *h_mask_bits, size_t mb_plane_stride, size_t mb_pitch,
+                                       uint8_t *h_edge_bits, size_t eb_plane_stride, size_t eb_pitch, int bit_order,
+                                       int64_t *h_counts);
 
 /* Non-zero count of each of K planes (02:157, 03:38 `np.count_nonzero`); h_counts: K int64.
  * Synchronises the stream. */

@@ -482,22 +482,40 @@ extern "C" int omni_layer_masks(omni_ctx *ctx, const uint8_t *d_labels, int h, i
 }
 
 // opt-in: the Lab centres of 02_color_extract.py:39-50 on the device (see kmeans.cu for the contract)
+static int kmeans_checked(const char *fn, omni_ctx *ctx, const uint8_t *d_bgr, int n_frames, size_t frame_stride, int h, int w, size_t pitch,
+                          const int32_t *h_sample_idx, int n_samples, int K, int attempts, int max_iter, double eps, uint64_t seed,
+                          float *h_centers, double *h_compactness, void *stream)
+{
+    OMNI_TRY(set_device(ctx));
+    OMNI_REQUIRE(d_bgr && h_centers, "%s: NULL pointer", fn);
+    OMNI_REQUIRE(h > 0 && w > 0 && pitch >= (size_t)w * 3 && (long long)h * w < (1ll << 31), "%s: bad geometry", fn);
+    OMNI_REQUIRE(n_frames >= 1 && (n_frames == 1 || frame_stride >= pitch * (size_t)(h - 1) + (size_t)w * 3),
+                 "%s: %d frames, frame_stride %zu smaller than a frame", fn, n_frames, frame_stride);
+    OMNI_REQUIRE(K >= 1 && K <= OMNI_MAX_K, "%s: K=%d outside [1,%d]", fn, K, OMNI_MAX_K);
+    OMNI_REQUIRE(attempts >= 1 && attempts <= 64 && max_iter >= 1 && max_iter <= 1000 && eps >= 0.0, "%s: bad criteria", fn);
+    const int n = h_sample_idx ? n_samples : h * w;
+    OMNI_REQUIRE(n >= K && n <= (1 << 24), "%s: %d samples (need K <= n <= 2^24: integer accumulators)", fn, n);
+    if (h_sample_idx)
+        for (int i = 0; i < n; i++)
+            OMNI_REQUIRE(h_sample_idx[i] >= 0 && h_sample_idx[i] < h * w, "%s: sample index %d out of range", fn, h_sample_idx[i]);
+    return kmeans_lab_batch(ctx, d_bgr, n_frames, frame_stride, h, w, pitch, h_sample_idx, n, K, attempts, max_iter, (float)eps,
+                            (unsigned long long)seed, h_centers, h_compactness, (cudaStream_t)stream);
+}
+
 extern "C" int omni_kmeans_lab(omni_ctx *ctx, const uint8_t *d_bgr, int h, int w, size_t pitch, const int32_t *h_sample_idx, int n_samples,
                                int K, int attempts, int max_iter, double eps, uint64_t seed, float *h_centers, double *h_compactness,
                                void *stream)
 {
-    OMNI_TRY(set_device(ctx));
-    OMNI_REQUIRE(d_bgr && h_centers, "omni_kmeans_lab: NULL pointer");
-    OMNI_REQUIRE(h > 0 && w > 0 && pitch >= (size_t)w * 3 && (long long)h * w < (1ll << 31), "omni_kmeans_lab: bad geometry");
-    OMNI_REQUIRE(K >= 1 && K <= OMNI_MAX_K, "omni_kmeans_lab: K=%d outside [1,%d]", K, OMNI_MAX_K);
-    OMNI_REQUIRE(attempts >= 1 && attempts <= 64 && max_iter >= 1 && max_iter <= 1000 && eps >= 0.0, "omni_kmeans_lab: bad criteria");
-    const int n = h_sample_idx ? n_samples : h * w;
-    OMNI_REQUIRE(n >= K && n <= (1 << 24), "omni_kmeans_lab: %d samples (need K <= n <= 2^24: integer accumulators)", n);
-    if (h_sample_idx)
-        for (int i = 0; i < n; i++)
-            OMNI_REQUIRE(h_sample_idx[i] >= 0 && h_sample_idx[i] < h * w, "omni_kmeans_lab: sample index %d out of range", h_sample_idx[i]);
-    return kmeans_lab(ctx, d_bgr, h, w, pitch, h_sample_idx, n, K, attempts, max_iter, (float)eps, (unsigned long long)seed, h_centers,
-                      h_compactness, (cudaStream_t)stream);
+    return kmeans_checked("omni_kmeans_lab", ctx, d_bgr, 1, 0, h, w, pitch, h_sample_idx, n_samples, K, attempts, max_iter, eps, seed,
+                          h_centers, h_compactness, stream);
+}
+
+extern "C" int omni_kmeans_lab_batch(omni_ctx *ctx, const uint8_t *d_bgr, int n_frames, size_t frame_stride, int h, int w, size_t pitch,
+                                     const int32_t *h_sample_idx, int n_samples, int K, int attempts, int max_iter, double eps, uint64_t seed,
+                                     float *h_centers, double *h_compactness, void *stream)
+{
+    return kmeans_checked("omni_kmeans_lab_batch", ctx, d_bgr, n_frames, frame_stride, h, w, pitch, h_sample_idx, n_samples, K, attempts,
+                          max_iter, eps, seed, h_centers, h_compactness, stream);
 }
 
 // ---- stage 03 ----------------------------------------------------------------------------------------
@@ -677,11 +695,12 @@ extern "C" int omni_color_edge_batch(omni_ctx *ctx, const uint8_t *d_bgr, int n_
 static inline size_t pad16(size_t v) { return (v + 15) & ~(size_t)15; }
 
 // ---- packed (1 bit per pixel) outputs ------------------------------------------------------------------------
-// Device body shared by the three packed entry points: n frames at d_bgr -> packed planes (device, caller layout) + counts on
-// the device (ctx->d_counts: [pixels | mask non-zeros | edge non-zeros], OMNI_MAX_K each) when want_counts.
+// Device body shared by the packed entry points: n frames at d_bgr -> packed planes (device, caller layout) + counts on the device
+// (ctx->d_counts: [pixels | mask non-zeros | edge non-zeros], OMNI_MAX_K each) when want_counts.  per_frame: frame f has its own
+// centres h_centers + f * K * 3 and LUT h_lut + f * K (else all frames share h_centers / h_lut).
 static int packed_device(omni_ctx *ctx, const u8 *d_bgr, int nf, size_t frame_stride, int h, int w, size_t pitch, const float *h_centers,
                          int K, const uint8_t *h_lut, const omni_edge_params *prm, u8 *d_mb, size_t mb_plane, size_t mb_pitch,
-                         u8 *d_eb, size_t eb_plane, size_t eb_pitch, int bit_order, bool want_counts, cudaStream_t st)
+                         u8 *d_eb, size_t eb_plane, size_t eb_pitch, int bit_order, bool want_counts, cudaStream_t st, bool per_frame = false)
 {
     OMNI_REQUIRE(bit_order == OMNI_BITS_LSB_FIRST || bit_order == OMNI_BITS_MSB_FIRST, "bit_order must be OMNI_BITS_LSB_FIRST or OMNI_BITS_MSB_FIRST");
     OMNI_REQUIRE(nf >= 1 && nf * K <= OMNI_MAX_K, "n_frames * K = %d exceeds %d planes per call", nf * K, OMNI_MAX_K);
@@ -689,13 +708,16 @@ static int packed_device(omni_ctx *ctx, const u8 *d_bgr, int nf, size_t frame_st
     OMNI_REQUIRE(mb_pitch >= rb && (!prm || eb_pitch >= rb), "packed row pitch smaller than ceil(w / 8) bytes");
     BlurParams bp; int low = 0, high = 0;
     if (prm) OMNI_TRY(check_edge_params(prm, &bp, &low, &high));
-    AssignParams P;
+    const size_t cs = per_frame ? (size_t)3 * K : 0, ls = per_frame ? (size_t)K : 0;     // centre / LUT stride between frames
+    AssignParams P, Pf[OMNI_MAX_K];
     OMNI_TRY(fill_assign(&P, h_centers, nullptr, K, h_lut));
+    if (per_frame)
+        for (int f = 0; f < nf; f++) OMNI_TRY(fill_assign(&Pf[f], h_centers + f * cs, nullptr, K, h_lut ? h_lut + f * ls : nullptr));
     unsigned long long *dc = want_counts ? ctx->d_counts : nullptr;
     int rc = OMNI_ERR_UNSUPPORTED;
     if (ctx->fast && ctx->pipeline == 1)
         rc = label_color_edge_packed(ctx, d_bgr, nf, frame_stride, h, w, pitch, P, prm, low, high, d_mb, mb_plane, mb_pitch, d_eb, eb_plane,
-                                     eb_pitch, bit_order == OMNI_BITS_MSB_FIRST, dc, st);
+                                     eb_pitch, bit_order == OMNI_BITS_MSB_FIRST, dc, st, per_frame ? Pf : nullptr);
     if (rc != OMNI_ERR_UNSUPPORTED) return rc;
     // any other family: byte planes in workspace slot 2, then packed
     const size_t bp_pitch = ((size_t)w + 15) & ~(size_t)15, bplane = bp_pitch * h, lp = bp_pitch;
@@ -706,12 +728,14 @@ static int packed_device(omni_ctx *ctx, const u8 *d_bgr, int nf, size_t frame_st
     omni_edge_params none{1, 0, 0, 3, 50.0, 150.0};          // masks only: the edge planes of a cheap dummy pass are dropped
     for (int f = 0; f < nf; f++) {
         const u8 *img = d_bgr + (size_t)f * frame_stride;
+        const float *ctr = h_centers + f * cs;
+        const uint8_t *lut = h_lut ? h_lut + f * ls : nullptr;
         if (prm) {
-            OMNI_TRY(omni_color_edge(ctx, img, h, w, pitch, h_centers, K, h_lut, prm, dl, lp, dm + (size_t)f * K * bplane, bplane, bp_pitch,
+            OMNI_TRY(omni_color_edge(ctx, img, h, w, pitch, ctr, K, lut, prm, dl, lp, dm + (size_t)f * K * bplane, bplane, bp_pitch,
                                      de + (size_t)f * K * bplane, bplane, bp_pitch, st));
         } else {
             (void)none;
-            OMNI_TRY(omni_assign_lab_f32(ctx, img, h, w, pitch, h_centers, K, h_lut, dl, lp, st));
+            OMNI_TRY(omni_assign_lab_f32(ctx, img, h, w, pitch, ctr, K, lut, dl, lp, st));
             OMNI_TRY(omni_layer_masks(ctx, dl, h, w, lp, K, 1, 1, dm + (size_t)f * K * bplane, bplane, bp_pitch, st));
         }
         if (dc) OMNI_LAUNCH(ctx, st, "count_labels", g_count_labels(dl, lp, h, w, K, dc + (size_t)f * K, st));
@@ -731,18 +755,18 @@ static void fetch_counts(omni_ctx *ctx, int KT, int64_t *h_counts)
     }
 }
 
-extern "C" int omni_color_edge_packed(omni_ctx *ctx, const uint8_t *d_bgr, int n_frames, size_t frame_stride, int h, int w, size_t pitch,
-                                      const float *h_centers, int K, const uint8_t *h_lut, const omni_edge_params *prm,
-                                      uint8_t *d_mask_bits, size_t mb_plane_stride, size_t mb_pitch,
-                                      uint8_t *d_edge_bits, size_t eb_plane_stride, size_t eb_pitch, int bit_order,
-                                      int64_t *h_counts, void *stream)
+static int device_packed(const char *fn, omni_ctx *ctx, const uint8_t *d_bgr, int n_frames, size_t frame_stride, int h, int w, size_t pitch,
+                         const float *h_centers, int K, const uint8_t *h_lut, const omni_edge_params *prm,
+                         uint8_t *d_mask_bits, size_t mb_plane_stride, size_t mb_pitch,
+                         uint8_t *d_edge_bits, size_t eb_plane_stride, size_t eb_pitch, int bit_order,
+                         int64_t *h_counts, void *stream, bool per_frame)
 {
     OMNI_TRY(set_device(ctx));
-    OMNI_REQUIRE(d_bgr && d_mask_bits && h_centers && (d_edge_bits || !prm), "omni_color_edge_packed: NULL pointer");
-    OMNI_REQUIRE(h > 0 && w > 0 && pitch >= (size_t)w * 3 && K >= 1 && K <= OMNI_MAX_K, "omni_color_edge_packed: bad geometry");
+    OMNI_REQUIRE(d_bgr && d_mask_bits && h_centers && (d_edge_bits || !prm), "%s: NULL pointer", fn);
+    OMNI_REQUIRE(h > 0 && w > 0 && pitch >= (size_t)w * 3 && K >= 1 && K <= OMNI_MAX_K, "%s: bad geometry", fn);
     cudaStream_t st = (cudaStream_t)stream;
     OMNI_TRY(packed_device(ctx, d_bgr, n_frames, frame_stride, h, w, pitch, h_centers, K, h_lut, prm, d_mask_bits, mb_plane_stride, mb_pitch,
-                           d_edge_bits, eb_plane_stride, eb_pitch, bit_order, h_counts != nullptr, st));
+                           d_edge_bits, eb_plane_stride, eb_pitch, bit_order, h_counts != nullptr, st, per_frame));
     if (h_counts) {
         OMNI_CUDA(cudaMemcpyAsync(ctx->h_counts, ctx->d_counts, 3 * OMNI_MAX_K * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
         OMNI_CUDA(cudaStreamSynchronize(st));
@@ -751,21 +775,47 @@ extern "C" int omni_color_edge_packed(omni_ctx *ctx, const uint8_t *d_bgr, int n
     return OMNI_OK;
 }
 
-// Host buffers, n frames sharing one centre set, H2D / kernels / D2H of consecutive frame groups overlapped (two staging slots on
-// three streams).  Results are complete in the host buffers when the call returns.
-extern "C" int omni_host_color_edge_packed(omni_ctx *ctx, const uint8_t *h_bgr, int n_frames, size_t frame_stride, int h, int w, size_t pitch,
-                                           const float *h_centers, int K, const uint8_t *h_lut, const omni_edge_params *prm,
-                                           uint8_t *h_mask_bits, size_t mb_plane_stride, size_t mb_pitch,
-                                           uint8_t *h_edge_bits, size_t eb_plane_stride, size_t eb_pitch, int bit_order,
-                                           int64_t *h_counts)
+extern "C" int omni_color_edge_packed(omni_ctx *ctx, const uint8_t *d_bgr, int n_frames, size_t frame_stride, int h, int w, size_t pitch,
+                                      const float *h_centers, int K, const uint8_t *h_lut, const omni_edge_params *prm,
+                                      uint8_t *d_mask_bits, size_t mb_plane_stride, size_t mb_pitch,
+                                      uint8_t *d_edge_bits, size_t eb_plane_stride, size_t eb_pitch, int bit_order,
+                                      int64_t *h_counts, void *stream)
+{
+    return device_packed("omni_color_edge_packed", ctx, d_bgr, n_frames, frame_stride, h, w, pitch, h_centers, K, h_lut, prm, d_mask_bits,
+                         mb_plane_stride, mb_pitch, d_edge_bits, eb_plane_stride, eb_pitch, bit_order, h_counts, stream, false);
+}
+
+extern "C" int omni_color_edge_packed_frames(omni_ctx *ctx, const uint8_t *d_bgr, int n_frames, size_t frame_stride, int h, int w, size_t pitch,
+                                             const float *h_centers, int K, const uint8_t *h_luts, const omni_edge_params *prm,
+                                             uint8_t *d_mask_bits, size_t mb_plane_stride, size_t mb_pitch,
+                                             uint8_t *d_edge_bits, size_t eb_plane_stride, size_t eb_pitch, int bit_order,
+                                             int64_t *h_counts, void *stream)
+{
+    return device_packed("omni_color_edge_packed_frames", ctx, d_bgr, n_frames, frame_stride, h, w, pitch, h_centers, K, h_luts, prm,
+                         d_mask_bits, mb_plane_stride, mb_pitch, d_edge_bits, eb_plane_stride, eb_pitch, bit_order, h_counts, stream, true);
+}
+
+// Host buffers, n frames sharing one centre set (or, per_frame, each with its own), H2D / kernels / D2H of consecutive frame groups
+// overlapped (two staging slots on three streams).  Results are complete in the host buffers when the call returns.
+static int host_packed(const char *fn, omni_ctx *ctx, const uint8_t *h_bgr, int n_frames, size_t frame_stride, int h, int w, size_t pitch,
+                       const float *h_centers, int K, const uint8_t *h_lut, const omni_edge_params *prm,
+                       uint8_t *h_mask_bits, size_t mb_plane_stride, size_t mb_pitch,
+                       uint8_t *h_edge_bits, size_t eb_plane_stride, size_t eb_pitch, int bit_order,
+                       int64_t *h_counts, bool per_frame)
 {
     OMNI_TRY(set_device(ctx));
-    OMNI_REQUIRE(h_bgr && h_mask_bits && h_centers && (h_edge_bits || !prm) && n_frames >= 1, "omni_host_color_edge_packed: bad arguments");
-    OMNI_REQUIRE(h > 0 && w > 0 && pitch >= (size_t)w * 3 && K >= 1 && K <= OMNI_MAX_K, "omni_host_color_edge_packed: bad geometry");
+    OMNI_REQUIRE(h_bgr && h_mask_bits && h_centers && (h_edge_bits || !prm) && n_frames >= 1, "%s: bad arguments", fn);
+    OMNI_REQUIRE(h > 0 && w > 0 && pitch >= (size_t)w * 3 && K >= 1 && K <= OMNI_MAX_K, "%s: bad geometry", fn);
     const size_t rb = ((size_t)w + 7) / 8;
     OMNI_REQUIRE(mb_pitch >= rb && (!prm || eb_pitch >= rb), "packed row pitch smaller than ceil(w / 8) bytes");
     OMNI_REQUIRE(mb_plane_stride == mb_pitch * (size_t)h && (!prm || eb_plane_stride == eb_pitch * (size_t)h),
-                 "omni_host_color_edge_packed: planes must be back to back (plane stride = pitch * h)");
+                 "%s: planes must be back to back (plane stride = pitch * h)", fn);
+    if (per_frame) {                                        // every frame's LUT before any work, as fill_assign checks it
+        AssignParams P;
+        for (int f = 0; f < n_frames; f++)
+            OMNI_TRY(fill_assign(&P, h_centers + (size_t)f * 3 * K, nullptr, K, h_lut ? h_lut + (size_t)f * K : nullptr));
+    }
+    const size_t cs = per_frame ? (size_t)3 * K : 0, ls = per_frame ? (size_t)K : 0;     // centre / LUT stride between frames
     const int G = OMNI_MAX_K / K;                           // frames per device pass (their G * K layers are its planes)
     const int n_groups = (n_frames + G - 1) / G;
     if (!ctx->pk_ready) {
@@ -810,8 +860,8 @@ extern "C" int omni_host_color_edge_packed(omni_ctx *ctx, const uint8_t *h_bgr, 
         OMNI_CUDA(cudaEventRecord(ctx->pk_ev[s], si));
         OMNI_CUDA(cudaStreamWaitEvent(sc, ctx->pk_ev[s], 0));
         if (gi >= 2) OMNI_CUDA(cudaStreamWaitEvent(sc, ctx->pk_ev[4 + s], 0));      // the D2H of group gi-2 has drained this slot's outputs
-        OMNI_TRY(packed_device(ctx, d_in, nf, img_bytes, h, w, ip, h_centers, K, h_lut, prm, d_mb, dplane, dp, d_eb, dplane, dp, bit_order,
-                               h_counts != nullptr, sc));
+        OMNI_TRY(packed_device(ctx, d_in, nf, img_bytes, h, w, ip, h_centers + f0 * cs, K, h_lut ? h_lut + f0 * ls : nullptr, prm, d_mb, dplane,
+                               dp, d_eb, dplane, dp, bit_order, h_counts != nullptr, sc, per_frame));
         if (h_counts)
             OMNI_CUDA(cudaMemcpyAsync(ctx->pk_counts + (size_t)gi * 3 * OMNI_MAX_K, ctx->d_counts, 3 * OMNI_MAX_K * sizeof(unsigned long long),
                                       cudaMemcpyDeviceToHost, sc));
@@ -837,6 +887,26 @@ extern "C" int omni_host_color_edge_packed(omni_ctx *ctx, const uint8_t *h_bgr, 
             }
         }
     return OMNI_OK;
+}
+
+extern "C" int omni_host_color_edge_packed(omni_ctx *ctx, const uint8_t *h_bgr, int n_frames, size_t frame_stride, int h, int w, size_t pitch,
+                                           const float *h_centers, int K, const uint8_t *h_lut, const omni_edge_params *prm,
+                                           uint8_t *h_mask_bits, size_t mb_plane_stride, size_t mb_pitch,
+                                           uint8_t *h_edge_bits, size_t eb_plane_stride, size_t eb_pitch, int bit_order,
+                                           int64_t *h_counts)
+{
+    return host_packed("omni_host_color_edge_packed", ctx, h_bgr, n_frames, frame_stride, h, w, pitch, h_centers, K, h_lut, prm, h_mask_bits,
+                       mb_plane_stride, mb_pitch, h_edge_bits, eb_plane_stride, eb_pitch, bit_order, h_counts, false);
+}
+
+extern "C" int omni_host_color_edge_packed_frames(omni_ctx *ctx, const uint8_t *h_bgr, int n_frames, size_t frame_stride, int h, int w,
+                                                  size_t pitch, const float *h_centers, int K, const uint8_t *h_luts,
+                                                  const omni_edge_params *prm, uint8_t *h_mask_bits, size_t mb_plane_stride, size_t mb_pitch,
+                                                  uint8_t *h_edge_bits, size_t eb_plane_stride, size_t eb_pitch, int bit_order,
+                                                  int64_t *h_counts)
+{
+    return host_packed("omni_host_color_edge_packed_frames", ctx, h_bgr, n_frames, frame_stride, h, w, pitch, h_centers, K, h_luts, prm,
+                       h_mask_bits, mb_plane_stride, mb_pitch, h_edge_bits, eb_plane_stride, eb_pitch, bit_order, h_counts, true);
 }
 
 // ---- counts / composite -----------------------------------------------------------------------------------

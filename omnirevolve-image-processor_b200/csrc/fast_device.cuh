@@ -196,8 +196,9 @@ cudaError_t launch_pack_planes(const u32 *src, int ws, size_t plane, int K, int 
 void dense_ws_bytes(int h, int w, int K, int nf, int ksize, size_t out[OMNI_WS_SLOTS]);   // fast_kernels.cu
 
 // opt-in device k-means of the Lab centres (kmeans.cu)
-int kmeans_lab(omni_ctx *ctx, const u8 *d_bgr, int h, int w, size_t pitch, const int *h_idx, int n, int K, int attempts, int max_iter,
-               float eps, unsigned long long seed, float *h_centers, double *h_compactness, cudaStream_t st);
+int kmeans_lab_batch(omni_ctx *ctx, const u8 *d_bgr, int n_frames, size_t frame_stride, int h, int w, size_t pitch, const int *h_idx,
+                     int n, int K, int attempts, int max_iter, float eps, unsigned long long seed, float *h_centers,
+                     double *h_compactness, cudaStream_t st);
 
 // sparse generation of the fused colour+edge call (label_pipe.cu); OMNI_ERR_UNSUPPORTED: use the dense generation
 int sparse_color_edge(omni_ctx *ctx, const u8 *d_bgr, int nf, size_t frame_stride, int h, int w, size_t pitch, const AssignParams &P,

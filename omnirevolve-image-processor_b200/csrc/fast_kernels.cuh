@@ -84,10 +84,12 @@ int fast_color_edge_batch(omni_ctx *ctx, const u8 *d_bgr, int n, size_t frame_st
                           const omni_edge_params *prm, int low, int high, u8 *d_masks, size_t m_plane, size_t mpitch,
                           u8 *d_edges, size_t e_plane, size_t epitch, cudaStream_t st);
 
-// packed (1 bit per pixel) outputs of the fused call (label_pipe.cu); prm == NULL: colour layers only
+// packed (1 bit per pixel) outputs of the fused call (label_pipe.cu); prm == NULL: colour layers only; Pf != NULL: frame f assigned
+// with Pf[f] (nf sets, K = P.K) instead of P
 int label_color_edge_packed(omni_ctx *ctx, const u8 *d_bgr, int nf, size_t frame_stride, int h, int w, size_t pitch, const AssignParams &P,
                             const omni_edge_params *prm, int low, int high, u8 *d_mask_bits, size_t mb_plane, size_t mb_pitch,
-                            u8 *d_edge_bits, size_t eb_plane, size_t eb_pitch, int msb_first, unsigned long long *d_counts, cudaStream_t st);
+                            u8 *d_edge_bits, size_t eb_plane, size_t eb_pitch, int msb_first, unsigned long long *d_counts, cudaStream_t st,
+                            const AssignParams *Pf = nullptr);
 // one image in HOST memory, row bands pipelined (H2D of band b+1 | kernels of band b | D2H of band b-1); OMNI_ERR_UNSUPPORTED: not
 // applicable (small image, outside the label pipeline) -- the caller takes the frame-group path
 int label_host_packed_banded(omni_ctx *ctx, const u8 *h_bgr, int h, int w, size_t pitch, const AssignParams &P, const omni_edge_params *prm,

@@ -763,16 +763,21 @@ static cudaError_t launch_open_morph(int kind /* -1: masks only */, const uint4 
 struct LabelPlanes { u32 *slices, *mask_bits, *edge_bits, *cand_bits; };
 
 // prm == NULL: colour layers only (02_color_extract.py on its own: no stage-03 work).  d_masks / d_edges may be NULL (packed
-// outputs: the bit-planes in `out` are the result).
+// outputs: the bit-planes in `out` are the result).  Pf (optional): nf centre sets, frame f assigned with Pf[f] (same K as P); the
+// frames then get one table build and one assignment launch each, and share every launch after the assignment.
 static int label_pipeline(omni_ctx *ctx, const u8 *d_bgr, int nf, size_t frame_stride, int h, int w, size_t pitch, const AssignParams &P,
                           const omni_edge_params *prm, int low, int high, u8 *d_labels, size_t lpitch,
                           u8 *d_masks, size_t m_plane, size_t mpitch, u8 *d_edges, size_t e_plane, size_t epitch, bool want_mask_bits,
-                          cudaStream_t st, LabelPlanes *out, bool skip_hysteresis = false /* bands: S and C are the result */)
+                          cudaStream_t st, LabelPlanes *out, bool skip_hysteresis = false /* bands: S and C are the result */,
+                          const AssignParams *Pf = nullptr)
 {
     const int K = P.K, KT = nf * K;
     const int kind = prm ? morph03_kind(prm) : -1;
     if (prm && (low < 0 || kind < 0 || prm->ksize != 3)) return OMNI_ERR_UNSUPPORTED;
     if (K > RC_MAX_K || KT > OMNI_MAX_K || !lut_below_k(P) || !edges3_sparse_ok(h, w, KT)) return OMNI_ERR_UNSUPPORTED;
+    if (Pf)
+        for (int f = 0; f < nf; f++)
+            if (Pf[f].K != K || !lut_below_k(Pf[f])) return OMNI_ERR_UNSUPPORTED;
     const BitGeom g = make_geom(h, w);
     if ((long long)nf * h * ((w + 255) >> 8) >= (1ll << 30)) return OMNI_ERR_UNSUPPORTED;
     OMNI_CUDA(fast_tables());
@@ -795,29 +800,38 @@ static int label_pipeline(omni_ctx *ctx, const u8 *d_bgr, int nf, size_t frame_s
         SP_TRY(edge_pass_begin(ctx, g, KT, sbits, cbits, d_edges, e_plane, epitch, st, &R, &sparse, d_edges != nullptr, d_edges ? &Z : nullptr));
         if (!sparse) return OMNI_ERR_UNSUPPORTED;
     }
-    u32 *cells = nullptr;
-    u8 *rtab = nullptr;
-    SP_TRY(label_tables(ctx, P, &cells, &rtab, st));
     const u16 *labtab = fast_lab_table();
     if (!labtab) { omni_set_error("Lab tables not available"); return OMNI_ERR_CUDA; }
-    // ---- 1. assignment -> label bit-slices ----
-    {
-        if (!ctx->occ_assign_sl) {
-            OMNI_CUDA(cudaFuncSetAttribute(fk_assign_slices<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, RA_SMEM + LP_ZBUF));
-            OMNI_CUDA(cudaFuncSetAttribute(fk_assign_slices<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, RA_SMEM + LP_ZBUF));
-            ctx->occ_assign_sl = 1;
-        }
-        const long long chunks = (long long)nf * h * ((w + 255) >> 8);
+    // ---- 1. assignment -> label bit-slices: all frames in one launch, or (Pf) one table build + launch per frame ----
+    if (!ctx->occ_assign_sl) {
+        OMNI_CUDA(cudaFuncSetAttribute(fk_assign_slices<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, RA_SMEM + LP_ZBUF));
+        OMNI_CUDA(cudaFuncSetAttribute(fk_assign_slices<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, RA_SMEM + LP_ZBUF));
+        ctx->occ_assign_sl = 1;
+    }
+    for (int f0 = 0, n_in = Pf ? 1 : nf; f0 < nf; f0 += n_in) {
+        const AssignParams &Pa = Pf ? Pf[f0] : P;
+        u32 *cells = nullptr;
+        u8 *rtab = nullptr;
+        SP_TRY(label_tables(ctx, Pa, &cells, &rtab, st));
+        const long long chunks = (long long)n_in * h * ((w + 255) >> 8);
         const int grid = (int)std::max<long long>(1, std::min<long long>(persist_blocks(ctx, 1), (chunks + RA_WARPS - 1) / RA_WARPS));
-        for (int z = 0; z < 2; z++)                         // units per chunk, rounded up to one store per lane
-            Z.per[z] = (unsigned)(((Z.n16[z] + (unsigned long long)chunks - 1) / (unsigned long long)chunks + 31) & ~31ull);
+        // the zero fill rides on the first launch only, spread over that launch's chunks
+        ZeroJob Za{};
+        if (f0 == 0) {
+            Za = Z;
+            for (int z = 0; z < 2; z++)                     // units per chunk, rounded up to one store per lane
+                Za.per[z] = (unsigned)(((Za.n16[z] + (unsigned long long)chunks - 1) / (unsigned long long)chunks + 31) & ~31ull);
+        }
+        const u8 *px = d_bgr + (size_t)f0 * frame_stride;
+        u8 *lab = d_labels ? d_labels + (size_t)f0 * h * lpitch : nullptr;
+        u32 *sl = slices + (size_t)f0 * 4 * g.plane;
         KScope ks(ctx, "assign_bits", st);
         if (K >= 16)
-            fk_assign_slices<true><<<grid, RA_THREADS, RA_SMEM + LP_ZBUF, st>>>(d_bgr, h, w, pitch, P, (const uint4 *)rtab, cells, labtab, d_labels,
-                                                                                lpitch, slices, g.ws, nf, frame_stride, Z);
+            fk_assign_slices<true><<<grid, RA_THREADS, RA_SMEM + LP_ZBUF, st>>>(px, h, w, pitch, Pa, (const uint4 *)rtab, cells, labtab, lab,
+                                                                                lpitch, sl, g.ws, n_in, frame_stride, Za);
         else
-            fk_assign_slices<false><<<grid, RA_THREADS, RA_SMEM + LP_ZBUF, st>>>(d_bgr, h, w, pitch, P, (const uint4 *)rtab, cells, labtab, d_labels,
-                                                                                 lpitch, slices, g.ws, nf, frame_stride, Z);
+            fk_assign_slices<false><<<grid, RA_THREADS, RA_SMEM + LP_ZBUF, st>>>(px, h, w, pitch, Pa, (const uint4 *)rtab, cells, labtab, lab,
+                                                                                 lpitch, sl, g.ws, n_in, frame_stride, Za);
         OMNI_CUDA(cudaGetLastError());
     }
     // ---- 2. label-domain open and the rest of the morphology chain per plane, run lists for the edge kernel ----
@@ -962,16 +976,18 @@ __global__ void __launch_bounds__(256) fk_count_labels_sl(const uint4 *__restric
     if (lane < K && mine) atomicAdd(counts + lane, mine);
 }
 
-// Body of omni_color_edge_packed / omni_host_color_edge_packed* (capi.cu checks the arguments): nf frames sharing one centre set;
-// plane f * K + k of the outputs is layer k of frame f.  d_* outputs are DEVICE buffers in the caller's layout; d_counts (optional,
+// Body of omni_color_edge_packed[_frames] / omni_host_color_edge_packed[_frames] (capi.cu checks the arguments): nf frames sharing
+// the centre set P, or (Pf != NULL) frame f with its own set Pf[f]; plane f * K + k of the outputs is layer k of frame f.  d_* outputs are DEVICE buffers in the caller's layout; d_counts (optional,
 // device, 3 * OMNI_MAX_K u64: [0..) pixels per label, [OMNI_MAX_K..) mask non-zeros, [2 OMNI_MAX_K..) edge non-zeros per plane,
 // cleared here).  OMNI_ERR_UNSUPPORTED: outside the label pipeline (K > 16, edge_kernel_size != 3, ...).
 int label_color_edge_packed(omni_ctx *ctx, const u8 *d_bgr, int nf, size_t frame_stride, int h, int w, size_t pitch, const AssignParams &P,
                             const omni_edge_params *prm, int low, int high, u8 *d_mask_bits, size_t mb_plane, size_t mb_pitch,
-                            u8 *d_edge_bits, size_t eb_plane, size_t eb_pitch, int msb_first, unsigned long long *d_counts, cudaStream_t st)
+                            u8 *d_edge_bits, size_t eb_plane, size_t eb_pitch, int msb_first, unsigned long long *d_counts, cudaStream_t st,
+                            const AssignParams *Pf)
 {
     LabelPlanes L{};
-    SP_TRY(label_pipeline(ctx, d_bgr, nf, frame_stride, h, w, pitch, P, prm, low, high, nullptr, 0, nullptr, 0, 0, nullptr, 0, 0, true, st, &L));
+    SP_TRY(label_pipeline(ctx, d_bgr, nf, frame_stride, h, w, pitch, P, prm, low, high, nullptr, 0, nullptr, 0, 0, nullptr, 0, 0, true, st, &L,
+                          false, Pf));
     const BitGeom g = make_geom(h, w);
     const int K = P.K, KT = nf * K;
     if (d_counts) OMNI_CUDA(cudaMemsetAsync(d_counts, 0, 3 * OMNI_MAX_K * sizeof(unsigned long long), st));

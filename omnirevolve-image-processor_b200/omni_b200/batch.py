@@ -49,10 +49,15 @@ def gather_counts(local: dict, n_frames: int, K: int, dist=None) -> np.ndarray |
 
 def process_shard_packed(engine, frames, frame_ids, centers, lut, edge_cfg, mask_bits=None, edge_bits=None):
     """This rank's frames [n,H,W,3] (host, ideally pinned) through omni_host_color_edge_packed: the masks and edge planes of frame
-    j land in mask_bits / edge_bits [j*K:(j+1)*K] (1 bit per pixel); returns ({frame_id: counts[K,3]}, result dict) for gather_counts."""
+    j land in mask_bits / edge_bits [j*K:(j+1)*K] (1 bit per pixel); returns ({frame_id: counts[K,3]}, result dict) for gather_counts.
+    centers [K,3] / lut [K] are shared by all frames; centers [n,K,3] / lut [n,K] are this rank's frames' own (row j for frame j,
+    e.g. the rows frame_ids select from per-frame centres of the whole batch)."""
     ids = [int(i) for i in frame_ids]
     if not ids:
         return {}, None
-    K = np.asarray(centers).reshape(-1, 3).shape[0]
+    c = np.asarray(centers)
+    K = c.shape[1] if c.ndim == 3 else c.reshape(-1, 3).shape[0]
+    if c.ndim == 3:
+        centers, lut = c[:len(ids)], None if lut is None else np.asarray(lut)[:len(ids)]
     r = engine.host_color_edge_packed(frames[:len(ids)], centers, lut, edge_cfg, mask_bits=mask_bits, edge_bits=edge_bits)
     return {f: r["counts"][j * K:(j + 1) * K] for j, f in enumerate(ids)}, r

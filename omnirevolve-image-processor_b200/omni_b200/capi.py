@@ -27,6 +27,7 @@ EXPORTS = [
     "omni_workspace_bytes", "omni_ctx_reserve", "omni_set_assume_binary_masks", "omni_kmeans_lab",
     "omni_thin_zhangsuen_packed", "omni_set_host_bands", "omni_last_band_resends",
     "omni_trace_centerlines", "omni_host_trace_centerlines", "omni_trace_results",
+    "omni_kmeans_lab_batch", "omni_color_edge_packed_frames", "omni_host_color_edge_packed_frames",
 ]
 
 
@@ -69,6 +70,7 @@ def lib():
         "omni_workspace_bytes": ([i, i, i, i, i], sz),
         "omni_ctx_reserve": ([vp, i, i, i, i, i], i),
         "omni_kmeans_lab": ([vp, u8p, i, i, sz, i32p, i, i, i, i, C.c_double, C.c_uint64, f32p, C.POINTER(C.c_double), vp], i),
+        "omni_kmeans_lab_batch": ([vp, u8p, i, sz, i, i, sz, i32p, i, i, i, i, C.c_double, C.c_uint64, f32p, C.POINTER(C.c_double), vp], i),
         "omni_ctx_create": ([i, C.POINTER(vp)], i),
         "omni_ctx_destroy": ([vp], i),
         "omni_host_alloc": ([sz, C.POINTER(vp)], i),
@@ -97,6 +99,8 @@ def lib():
         "omni_skeleton_degree": ([vp, u8p, i, i, i, sz, sz, u8p, sz, sz, u8p, sz, sz, vp], i),
         "omni_color_edge_packed": ([vp, u8p, i, sz, i, i, sz, f32p, i, hu8, epp, u8p, sz, sz, u8p, sz, sz, i, i64p, vp], i),
         "omni_host_color_edge_packed": ([vp, u8p, i, sz, i, i, sz, f32p, i, hu8, epp, u8p, sz, sz, u8p, sz, sz, i, i64p], i),
+        "omni_color_edge_packed_frames": ([vp, u8p, i, sz, i, i, sz, f32p, i, hu8, epp, u8p, sz, sz, u8p, sz, sz, i, i64p, vp], i),
+        "omni_host_color_edge_packed_frames": ([vp, u8p, i, sz, i, i, sz, f32p, i, hu8, epp, u8p, sz, sz, u8p, sz, sz, i, i64p], i),
         "omni_swatch_masks": ([vp, u8p, i, i, sz, i32p, i, i, u8p, sz, sz, i32p, vp], i),
         "omni_trace_centerlines": ([vp, u8p, i, i, i, sz, sz, i64p, vp], i),
         "omni_host_trace_centerlines": ([vp, u8p, i, i, i, sz, sz, i64p], i),

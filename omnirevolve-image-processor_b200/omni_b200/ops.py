@@ -76,6 +76,22 @@ def _u8p(a):
     return a.ctypes.data_as(C.POINTER(C.c_uint8)) if a is not None else None
 
 
+def _centers_luts(centers, lut, n: int):
+    """centers [K,3] (one set for all n frames) or [n,K,3] (one per frame), lut [K] / [n,K] or None ->
+    (ctr f32, lut u8 | None, K, per_frame)."""
+    c = np.asarray(centers, dtype=np.float32)
+    lut_a = None if lut is None else np.ascontiguousarray(lut, dtype=np.uint8)
+    if c.ndim != 3:
+        ctr = np.ascontiguousarray(c).reshape(-1, 3)
+        return ctr, lut_a, ctr.shape[0], False
+    if c.shape[0] != n or c.shape[2] != 3:
+        raise ValueError(f"per-frame centers must be [n_frames={n}, K, 3], got {list(c.shape)}")
+    K = c.shape[1]
+    if lut_a is not None and lut_a.shape != (n, K):
+        raise ValueError(f"per-frame lut must be [n_frames={n}, K={K}], got {list(lut_a.shape)}")
+    return np.ascontiguousarray(c), lut_a, K, True
+
+
 def _check_img(t: torch.Tensor, ch: int | None):
     if not (isinstance(t, torch.Tensor) and t.is_cuda and t.dtype == torch.uint8):
         raise TypeError("expected a CUDA uint8 tensor")
@@ -135,6 +151,26 @@ class Engine:
         capi.check(self._L.omni_kmeans_lab(self._h, bgr.data_ptr(), bgr.shape[0], bgr.shape[1], bgr.stride(0), idx_p, n, K, attempts,
                                            max_iter, float(eps), int(seed), _f32p(ctr), C.byref(comp), self._stream()))
         return ctr, float(comp.value)
+
+    def kmeans_lab_batch(self, frames: torch.Tensor, K: int, sample_idx=None, attempts: int = 3, max_iter: int = 40, eps: float = 0.5,
+                         seed: int = 0):
+        """kmeans_lab for every frame of frames [n,H,W,3] (CUDA uint8) in shared launches (omni_kmeans_lab_batch): (centers f32
+        [n,K,3], compactness f64 [n]), frame f bit-identical to kmeans_lab(frames[f], ...).  sample_idx: shared by all frames."""
+        if frames.dim() != 4 or frames.shape[3] != 3 or frames.dtype != torch.uint8 or not frames.is_cuda or frames.stride(3) != 1 \
+                or frames.stride(2) != 3:
+            raise ValueError("frames must be a CUDA uint8 tensor [n,H,W,3] with packed pixels")
+        n, h, w = frames.shape[:3]
+        ctr = np.empty((n, K, 3), np.float32)
+        comp = np.empty(n, np.float64)
+        if sample_idx is None:
+            idx_p, ns = None, 0
+        else:
+            idx = np.ascontiguousarray(sample_idx, dtype=np.int32)
+            idx_p, ns = idx.ctypes.data_as(C.POINTER(C.c_int32)), idx.size
+        capi.check(self._L.omni_kmeans_lab_batch(self._h, frames.data_ptr(), n, frames.stride(0), h, w, frames.stride(1), idx_p, ns, K,
+                                                 attempts, max_iter, float(eps), int(seed), _f32p(ctr),
+                                                 comp.ctypes.data_as(C.POINTER(C.c_double)), self._stream()))
+        return ctr, comp
 
     def reserve(self, h: int, w: int, K: int, ksize: int = 3, n_frames: int = 1) -> int:
         """Allocate the workspaces of the fused calls for this geometry now (omni_ctx_reserve); returns their size in bytes."""
@@ -264,22 +300,22 @@ class Engine:
                           want_counts: bool = False):
         """Packed form of color_edge / color_edge_batch: frames [H,W,3] or [n,H,W,3] (n * K <= 32) ->
         (mask_bits, edge_bits | None[, counts]) as CUDA uint8 tensors [n*K, H, ceil(W/8)], one BIT per pixel (msb_first: the
-        scanline format of a 1-bit PNG = numpy.packbits default).  ec=None: colour layers only (stage 02 on its own)."""
+        scanline format of a 1-bit PNG = numpy.packbits default).  ec=None: colour layers only (stage 02 on its own).
+        centers [K,3] / lut [K]: one set for all frames; centers [n,K,3] / lut [n,K]: frame f uses centers[f], lut[f]."""
         if frames.dim() == 3:
             frames = frames.unsqueeze(0)
         if frames.dim() != 4 or frames.shape[3] != 3 or frames.dtype != torch.uint8 or not frames.is_cuda or frames.stride(3) != 1 \
                 or frames.stride(2) != 3:
             raise ValueError("frames must be a CUDA uint8 tensor [n,H,W,3] (or [H,W,3]) with packed pixels")
-        ctr = np.ascontiguousarray(centers, dtype=np.float32).reshape(-1, 3)
-        K = ctr.shape[0]
-        lut_a = None if lut is None else np.ascontiguousarray(lut, dtype=np.uint8)
         n, h, w = frames.shape[:3]
+        ctr, lut_a, K, per_frame = _centers_luts(centers, lut, n)
+        fn = self._L.omni_color_edge_packed_frames if per_frame else self._L.omni_color_edge_packed
         rb = (w + 7) // 8
         mb = torch.empty((n * K, h, rb), dtype=torch.uint8, device=frames.device)
         eb = torch.empty((n * K, h, rb), dtype=torch.uint8, device=frames.device) if ec is not None else None
         counts = np.zeros((n * K, 3), np.int64) if want_counts else None
         p = ec.to_c() if ec is not None else None
-        capi.check(self._L.omni_color_edge_packed(
+        capi.check(fn(
             self._h, frames.data_ptr(), n, frames.stride(0), h, w, frames.stride(1), _f32p(ctr), K, _u8p(lut_a),
             C.byref(p) if p is not None else None, mb.data_ptr(), mb.stride(0), mb.stride(1),
             eb.data_ptr() if eb is not None else None, eb.stride(0) if eb is not None else 0, eb.stride(1) if eb is not None else 0,
@@ -289,18 +325,18 @@ class Engine:
 
     def host_color_edge_packed(self, frames: np.ndarray, centers, lut, ec: "EdgeConfig | None", msb_first: bool = True,
                                mask_bits: np.ndarray | None = None, edge_bits: np.ndarray | None = None, want_counts: bool = True):
-        """Host frames [n,H,W,3] (or one [H,W,3]) sharing one centre set -> dict(mask_bits, edge_bits, counts): uint8 arrays
-        [n*K, H, ceil(W/8)], one bit per pixel.  Any n: frame groups are pipelined through the device (H2D / kernels / D2H overlap).
+        """Host frames [n,H,W,3] (or one [H,W,3]) -> dict(mask_bits, edge_bits, counts): uint8 arrays [n*K, H, ceil(W/8)], one bit per
+        pixel.  centers [K,3] / lut [K]: one centre set for all frames; centers [n,K,3] / lut [n,K]: frame f uses centers[f], lut[f].
+        Any n: frame groups are pipelined through the device (H2D / kernels / D2H overlap).
         Pass pinned arrays (pinned_empty) for `frames`, `mask_bits`, `edge_bits` for full PCIe speed."""
         fr = np.asarray(frames)
         if fr.ndim == 3:
             fr = fr[None]
         if fr.dtype != np.uint8 or fr.ndim != 4 or fr.shape[3] != 3 or fr.strides[3] != 1 or fr.strides[2] != 3:
             fr = np.ascontiguousarray(fr, dtype=np.uint8)
-        ctr = np.ascontiguousarray(centers, dtype=np.float32).reshape(-1, 3)
-        K = ctr.shape[0]
-        lut_a = None if lut is None else np.ascontiguousarray(lut, dtype=np.uint8)
         n, h, w = fr.shape[:3]
+        ctr, lut_a, K, per_frame = _centers_luts(centers, lut, n)
+        fn = self._L.omni_host_color_edge_packed_frames if per_frame else self._L.omni_host_color_edge_packed
         rb = (w + 7) // 8
         if mask_bits is None:
             mask_bits = np.empty((n * K, h, rb), np.uint8)
@@ -311,7 +347,7 @@ class Engine:
                 raise ValueError("mask_bits / edge_bits must be C-contiguous uint8 [n*K, H, ceil(W/8)]")
         counts = np.zeros((n * K, 3), np.int64) if want_counts else None
         p = ec.to_c() if ec is not None else None
-        capi.check(self._L.omni_host_color_edge_packed(
+        capi.check(fn(
             self._h, fr.ctypes.data, n, fr.strides[0], h, w, fr.strides[1], _f32p(ctr), K, _u8p(lut_a),
             C.byref(p) if p is not None else None, mask_bits.ctypes.data, mask_bits.strides[0], mask_bits.strides[1],
             edge_bits.ctypes.data if edge_bits is not None else None, edge_bits.strides[0] if edge_bits is not None else 0,

@@ -83,19 +83,27 @@ def _ensure_bgr(img):
     return img
 
 
+def _sample_pick(n: int, sample_limit: int):
+    """02_color_extract.py:37-42: the seeded subsample (None: every pixel).  It depends on the pixel count only."""
+    return np.random.default_rng(42).choice(n, size=sample_limit, replace=False) if n > sample_limit else None
+
+
 def kmeans_lab_centers(img_bgr: np.ndarray, k: int, sample_limit: int = 200_000, attempts: int = 3) -> np.ndarray:
     """02_color_extract.py:35-50: centres from cv2.kmeans on the seeded <=200k-pixel Lab subsample.
     Only the sampled pixels are converted (cvtColor is per-pixel, so the values are the reference's)."""
-    h, w = img_bgr.shape[:2]
-    n = h * w
-    flat = img_bgr.reshape(-1, 3)
-    pick = np.random.default_rng(42).choice(n, size=sample_limit, replace=False) if n > sample_limit else None
+    pick = _sample_pick(img_bgr.shape[0] * img_bgr.shape[1], sample_limit)
     if os.environ.get("OMNI_B200_KMEANS", "").lower() == "gpu":
         # opt-in (SURVEY 8f rank 2): the same subsample, clustered on the device -- cv2.kmeans' own centres cannot be reproduced
         # (global RNG); the contract is their quality (include/omni_b200.h omni_kmeans_lab, tests/test_gpu_kmeans.py)
         import torch
         centers, _comp = get_engine().kmeans_lab(torch.from_numpy(np.ascontiguousarray(img_bgr)).cuda(), k, pick, attempts=attempts)
         return centers
+    return _host_kmeans(img_bgr, k, pick, attempts)
+
+
+def _host_kmeans(img_bgr: np.ndarray, k: int, pick, attempts: int) -> np.ndarray:
+    """The cv2.kmeans branch of kmeans_lab_centers on the subsample `pick` (None: every pixel)."""
+    flat = img_bgr.reshape(-1, 3)
     if pick is not None:
         flat = flat[pick]
     lab = cv2.cvtColor(np.ascontiguousarray(flat).reshape(-1, 1, 3), cv2.COLOR_BGR2LAB)
@@ -120,6 +128,56 @@ def darkness_lut(centers: np.ndarray):
     lut = np.zeros_like(order)
     lut[order] = np.arange(len(order))
     return order, lut
+
+
+def _kmeans_args(cfg):
+    """02_color_extract.py:66-80 as color_extract_main reads it: (K, sample_limit, attempts)."""
+    K = max(2, min(len(list(cfg.color_names)), int(getattr(cfg, "cluster_k", len(cfg.color_names)))))
+    return K, int(getattr(cfg, "kmeans_sample_limit", 200_000)), int(getattr(cfg, "kmeans_attempts", 3))
+
+
+def frame_centers(frames, cfg, mode: str = "host", threads: int | None = None, group: int = 64):
+    """Stage 02's centres for every frame of a batch, each frame clustered on its own as a stage-02 run of that frame would:
+    (centers f32 [n,K,3], luts u8 [n,K]) for Engine.host_color_edge_packed / color_edge_packed with per-frame centres.
+    frames: [n,H,W,3] BGR (or a sequence of such images for mode="host").  The darkness LUT is the reference's argsort (darkness_lut).
+      mode="host": exact.  Per frame cv2.setRNGSeed(0), then the cv2.kmeans expression of kmeans_lab_centers: the centres of a
+        fresh-process stage-02 run on that frame (SURVEY A.7).  OpenCV's RNG is per thread, so frames run on `threads` threads
+        (default: up to 8) with the same result as one after another.
+      mode="gpu": opt-in, omni_kmeans_lab's quality contract (include/omni_b200.h).  Frames go to the device `group` at a time,
+        one omni_kmeans_lab_batch call per group, all with the reference's subsample indices."""
+    K, limit, attempts = _kmeans_args(cfg)
+    n = len(frames)
+    if n == 0:
+        return np.empty((0, K, 3), np.float32), np.empty((0, K), np.uint8)
+    if mode == "host":
+        def one(img):
+            img = _ensure_bgr(np.asarray(img))
+            cv2.setRNGSeed(0)
+            return _host_kmeans(img, K, _sample_pick(img.shape[0] * img.shape[1], limit), attempts)
+        workers = max(1, min(n, threads if threads is not None else min(8, os.cpu_count() or 1)))
+        if workers == 1:
+            centers = [one(f) for f in frames]
+        else:
+            from concurrent.futures import ThreadPoolExecutor
+            with ThreadPoolExecutor(workers) as ex:
+                centers = list(ex.map(one, frames))
+        centers = np.stack(centers).astype(np.float32)
+    elif mode == "gpu":
+        import torch
+        fr = np.asarray(frames)
+        if fr.ndim != 4 or fr.shape[3] != 3 or fr.dtype != np.uint8:
+            raise ValueError("mode='gpu' needs frames as one uint8 array [n,H,W,3]")
+        pick = _sample_pick(fr.shape[1] * fr.shape[2], limit)
+        eng = get_engine()
+        parts = []
+        for g0 in range(0, n, group):
+            d = torch.from_numpy(np.ascontiguousarray(fr[g0:g0 + group])).cuda()
+            parts.append(eng.kmeans_lab_batch(d, K, pick, attempts=attempts)[0])
+        centers = np.concatenate(parts)
+    else:
+        raise ValueError(f"mode must be 'host' or 'gpu', got {mode!r}")
+    luts = np.stack([darkness_lut(c)[1] for c in centers]).astype(np.uint8)
+    return centers, luts
 
 
 def _lab_to_bgr(lab3) -> tuple:
@@ -171,13 +229,11 @@ def color_extract_main(cfg, img=None) -> dict:
         raise RuntimeError(f"Cannot read resized image: {path}")
     img = _ensure_bgr(img)
     names = list(cfg.color_names)
-    K_cfg = int(getattr(cfg, "cluster_k", len(names)))
-    K = max(2, min(len(names), K_cfg))
+    K, sample_limit, attempts = _kmeans_args(cfg)
     if str(getattr(cfg, "extraction_mode", "kmeans")).lower() == "swatch":
         _swatch_extract(cfg, img, names)
         return {}
-    centers = kmeans_lab_centers(img, K, sample_limit=int(getattr(cfg, "kmeans_sample_limit", 200_000)),
-                                 attempts=int(getattr(cfg, "kmeans_attempts", 3)))
+    centers = kmeans_lab_centers(img, K, sample_limit=sample_limit, attempts=attempts)
     order, lut = darkness_lut(centers)
     centers_sorted = centers[order]
     open_iters = int(getattr(cfg, "extract_open_iters", 1))
