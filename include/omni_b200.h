@@ -303,6 +303,37 @@ int omni_host_trace_centerlines(omni_ctx *ctx, const uint8_t *h_skel, int K, int
  * (left, top, width, height, area) plus the number of polylines of the component.  Sizes: the totals of h_plane_info. */
 int omni_trace_results(omni_ctx *ctx, int32_t *h_points, int32_t *h_path_len, int32_t *h_comp);
 
+/* ---- PNG files of stages 01-03, encoded on the device --------------------------------------- */
+/* Replaces the PNG encode of the files stages 01-03 write: cv2.imwrite of resized.png (01_resize.py:30), of mask.png
+ * (02_color_extract.py:156) and edges.png (03_edge_detect.py:37), and of edges_composite.png in save_edges_composite
+ * (03_edge_detect.py:60-111).  n images of one geometry, image i at src + i * src_stride, rows `pitch` bytes apart ->
+ * n complete, standard PNG files, written back to back into the output buffer; h_sizes (n int64) receives each file's size.
+ *   OMNI_PNG_GRAY1: packed rows in the OMNI_BITS_MSB_FIRST layout (ceil(w / 8) bytes used per row; unused bits of the last
+ *                   byte are ignored) -> colour type 0, bit depth 1, filter 0 on every row (mask.png / edges.png).
+ *   OMNI_PNG_BGR8:  u8 BGR, HWC as cv2 holds it -> colour type 2, bit depth 8, stored as RGB as cv2.imwrite stores it; each row
+ *                   takes the filter None, Sub or Up with the smallest sum of |signed byte|.
+ * Every file decodes (libpng, zlib) to exactly the source pixels, and the bytes depend on the pixels only: the same input gives
+ * the same file whatever the stream, the ctx or the calls made before.  The image data is deflated in segments of whole
+ * scanlines -- max(1, min(256, 61440 / (row bytes + 1))) rows, row bytes = ceil(w / 8) or 3 * w -- each compressed on its own
+ * (run-length matches at distance 1, dynamic or fixed Huffman codes or a stored block, whichever is smallest) and written as
+ * its own IDAT chunk.
+ * Limits: a scanline of at most OMNI_PNG_MAX_SCANLINE bytes (filter byte included: GRAY1 w <= 491512, BGR8 w <= 20479) and
+ * h <= OMNI_PNG_MAX_ROWS.  out_capacity must be at least n * omni_png_bound(h, w, format).  The output may not overlap the
+ * input.  Scratch: workspace slot 11 of the ctx (grown on demand; not covered by omni_workspace_bytes).
+ * The device form synchronises the stream (the sizes go to the host).  The host form copies the pixels in with one copy of the
+ * span they occupy, encodes on the ctx's own stream and copies out only the compressed bytes; it returns when h_out holds them.
+ * One call per stage (all K planes of a stage at once) keeps the GPU busy; calls on one ctx must not overlap. */
+#define OMNI_PNG_GRAY1 0          /* packed MSB-first rows -> grey, bit depth 1 */
+#define OMNI_PNG_BGR8 1           /* u8 BGR HWC            -> colour type 2, bit depth 8 */
+#define OMNI_PNG_MAX_SCANLINE 61440
+#define OMNI_PNG_MAX_ROWS (1 << 24)
+/* Worst-case bytes of one file (every segment a stored block, plus chunk overhead); 0 for bad arguments. */
+size_t omni_png_bound(int h, int w, int format);
+int omni_png_encode(omni_ctx *ctx, const uint8_t *d_src, int n, size_t src_stride, int h, int w, size_t pitch, int format,
+                    uint8_t *d_out, size_t out_capacity, int64_t *h_sizes, void *stream);
+int omni_host_png_encode(omni_ctx *ctx, const uint8_t *h_src, int n, size_t src_stride, int h, int w, size_t pitch, int format,
+                         uint8_t *h_out, size_t out_capacity, int64_t *h_sizes);
+
 /* Diagnostics of the last omni_edges / omni_color_edge call on this ctx: number of global
  * hysteresis passes that were needed (>= 1). */
 int omni_last_hysteresis_passes(omni_ctx *ctx);

@@ -12,7 +12,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB_DIR = os.path.join(HERE, "lib")
 LIB = os.path.join(LIB_DIR, "libomni_b200.so")
-SOURCES = ["capi.cu", "generic_kernels.cu", "fast_kernels.cu", "edges3.cu", "label_pipe.cu", "resize_tma.cu", "kmeans.cu", "trace.cu", "morph_ellipse.cu"]
+SOURCES = ["capi.cu", "generic_kernels.cu", "fast_kernels.cu", "edges3.cu", "label_pipe.cu", "resize_tma.cu", "kmeans.cu", "trace.cu", "morph_ellipse.cu", "png_encode.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "--fmad=false",                      # float paths must round every product and sum (SURVEY A.1, A.4)
               "-Xcompiler", "-fPIC,-fvisibility=default"]

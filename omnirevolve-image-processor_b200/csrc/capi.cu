@@ -1176,3 +1176,61 @@ extern "C" int omni_host_color_edge(omni_ctx *ctx, const uint8_t *h_bgr, int h, 
         }
     return OMNI_OK;
 }
+
+// ---- PNG files of stages 01-03 (png_encode.cu) --------------------------------------------------------------------------------
+extern "C" size_t omni_png_bound(int h, int w, int format)
+{
+    if ((format != OMNI_PNG_GRAY1 && format != OMNI_PNG_BGR8) || h < 1 || w < 1 || h > OMNI_PNG_MAX_ROWS) return 0;
+    const long long row = (format == OMNI_PNG_GRAY1 ? ((long long)w + 7) / 8 : 3LL * w) + 1;
+    if (row > OMNI_PNG_MAX_SCANLINE) return 0;
+    return png_file_bound(h, w, format);
+}
+
+static int png_check(const char *fn, int n, int h, int w, size_t pitch, int format, size_t out_capacity)
+{
+    OMNI_REQUIRE(format == OMNI_PNG_GRAY1 || format == OMNI_PNG_BGR8, "%s: unknown format %d (OMNI_PNG_GRAY1 = 0, OMNI_PNG_BGR8 = 1)",
+                 fn, format);
+    OMNI_REQUIRE(n >= 1, "%s: n must be at least 1 (got %d)", fn, n);
+    OMNI_REQUIRE(h >= 1 && w >= 1, "%s: h and w must be at least 1 (got %d x %d)", fn, w, h);
+    const long long row = format == OMNI_PNG_GRAY1 ? ((long long)w + 7) / 8 : 3LL * w;
+    OMNI_REQUIRE(row + 1 <= OMNI_PNG_MAX_SCANLINE,
+                 "%s: a row of %d pixels is over the encoder's limit of OMNI_PNG_MAX_SCANLINE = %d bytes per scanline (w <= %d for this format)",
+                 fn, w, OMNI_PNG_MAX_SCANLINE, format == OMNI_PNG_GRAY1 ? 8 * (OMNI_PNG_MAX_SCANLINE - 1) : (OMNI_PNG_MAX_SCANLINE - 1) / 3);
+    OMNI_REQUIRE(h <= OMNI_PNG_MAX_ROWS, "%s: h = %d is over the encoder's limit of OMNI_PNG_MAX_ROWS = %d rows", fn, h, OMNI_PNG_MAX_ROWS);
+    OMNI_REQUIRE(pitch >= (size_t)row, "%s: pitch %zu is shorter than a row (%lld bytes)", fn, pitch, row);
+    const long long nseg = ((long long)h + png_segment_rows(w, format) - 1) / png_segment_rows(w, format);
+    OMNI_REQUIRE(nseg * n <= INT32_MAX, "%s: %d images of %d rows are over the encoder's limit of 2^31 - 1 segments per call", fn, n, h);
+    const size_t need = (size_t)n * png_file_bound(h, w, format);
+    OMNI_REQUIRE(out_capacity >= need, "%s: out_capacity %zu is below n * omni_png_bound = %zu", fn, out_capacity, need);
+    return OMNI_OK;
+}
+
+extern "C" int omni_png_encode(omni_ctx *ctx, const uint8_t *d_src, int n, size_t src_stride, int h, int w, size_t pitch, int format,
+                               uint8_t *d_out, size_t out_capacity, int64_t *h_sizes, void *stream)
+{
+    OMNI_TRY(set_device(ctx));
+    OMNI_REQUIRE(d_src && d_out && h_sizes, "omni_png_encode: NULL pointer argument");
+    OMNI_TRY(png_check("omni_png_encode", n, h, w, pitch, format, out_capacity));
+    return png_encode_run(ctx, d_src, n, src_stride, h, w, pitch, format, d_out, h_sizes, (cudaStream_t)stream);
+}
+
+extern "C" int omni_host_png_encode(omni_ctx *ctx, const uint8_t *h_src, int n, size_t src_stride, int h, int w, size_t pitch, int format,
+                                    uint8_t *h_out, size_t out_capacity, int64_t *h_sizes)
+{
+    OMNI_TRY(set_device(ctx));
+    OMNI_REQUIRE(h_src && h_out && h_sizes, "omni_host_png_encode: NULL pointer argument");
+    OMNI_TRY(png_check("omni_host_png_encode", n, h, w, pitch, format, out_capacity));
+    const size_t row = format == OMNI_PNG_GRAY1 ? ((size_t)w + 7) / 8 : (size_t)w * 3;
+    // the span the pixels occupy goes over in one copy, with the caller's strides; the files come back in one copy of their bytes
+    const size_t span = (size_t)(n - 1) * src_stride + (size_t)(h - 1) * pitch + row;
+    const size_t in_bytes = pad16(span), out_bytes = (size_t)n * png_file_bound(h, w, format);
+    OMNI_TRY(omni_ws_reserve(ctx, 3, in_bytes + out_bytes));
+    u8 *d_in = (u8 *)ctx->ws[3], *d_out = d_in + in_bytes;
+    OMNI_CUDA(cudaMemcpyAsync(d_in, h_src, span, cudaMemcpyHostToDevice, ctx->stream));
+    OMNI_TRY(png_encode_run(ctx, d_in, n, src_stride, h, w, pitch, format, d_out, h_sizes, ctx->stream));
+    size_t total = 0;
+    for (int i = 0; i < n; i++) total += (size_t)h_sizes[i];
+    OMNI_CUDA(cudaMemcpyAsync(h_out, d_out, total, cudaMemcpyDeviceToHost, ctx->stream));
+    OMNI_CUDA(cudaStreamSynchronize(ctx->stream));
+    return OMNI_OK;
+}

@@ -56,12 +56,12 @@ struct ResizeTab {
     ResizeTabDev dev{};
 };
 
-#define OMNI_WS_SLOTS 11
+#define OMNI_WS_SLOTS 12
 struct omni_ctx {
     int device = 0;
     int fast = 1;
     // grow-only device scratch
-    void *ws[OMNI_WS_SLOTS] = {};          // 0-2 generic planes, 3 host staging, 4 bit-planes, 5 misc, 6 edge run lists, 7-10 trace.cu
+    void *ws[OMNI_WS_SLOTS] = {};          // 0-2 generic planes, 3 host staging, 4 bit-planes, 5 misc, 6 edge run lists, 7-10 trace.cu, 11 png_encode.cu
     size_t ws_bytes[OMNI_WS_SLOTS] = {};
     int *d_flags = nullptr;          // 64 ints of device flags / counters
     unsigned long long *d_counts = nullptr;   // 4*OMNI_MAX_K counters
@@ -141,6 +141,14 @@ int omni_ws_reserve(omni_ctx *ctx, int slot, size_t bytes);
 int trace_run(omni_ctx *ctx, const u8 *d_skel, int K, int h, int w, size_t plane_stride, size_t pitch, int64_t *h_info,
               cudaStream_t st);
 int trace_results(omni_ctx *ctx, int32_t *points, int32_t *path_len, int32_t *comp);
+// PNG encoder (png_encode.cu): a segment holds at most PNG_SEG_MAX filtered bytes (one stored block) and PNG_SEG_ROWS rows
+constexpr int PNG_SEG_MAX = 61440;
+constexpr int PNG_SEG_ROWS = 256;
+int png_segment_rows(int w, int fmt);
+size_t png_file_bound(int h, int w, int fmt);
+// n files into d_out (back to back, room for n * png_file_bound checked by the caller), sizes into h_sizes; synchronises st
+int png_encode_run(omni_ctx *ctx, const u8 *d_src, int n, size_t src_stride, int h, int w, size_t pitch, int fmt, u8 *d_out,
+                   int64_t *h_sizes, cudaStream_t st);
 const ResizeTab *omni_get_resize_tab(omni_ctx *ctx, int sh, int sw, int dh, int dw, cudaStream_t st);
 void omni_build_se(int shape_ellipse, int k, MorphSE *se);
 int omni_gauss_weights(int k, BlurParams *bp);

@@ -15,6 +15,9 @@ OMNI_MAX_MORPH_K = 255
 ERR_UNSUPPORTED = -3
 BITS_LSB_FIRST = 0      # pixel x = bit (x & 7) of byte x >> 3
 BITS_MSB_FIRST = 1      # pixel x = bit 7 - (x & 7): the scanline of a 1-bit PNG, numpy.packbits default
+PNG_GRAY1 = 0           # packed MSB-first rows -> 1-bit greyscale PNG
+PNG_BGR8 = 1            # u8 BGR HWC -> 8-bit RGB PNG
+PNG_MAX_SCANLINE = 61440
 
 EXPORTS = [
     "omni_version", "omni_last_error_string", "omni_device_count", "omni_set_fast_path", "omni_ctx_create",
@@ -28,6 +31,7 @@ EXPORTS = [
     "omni_thin_zhangsuen_packed", "omni_set_host_bands", "omni_last_band_resends",
     "omni_trace_centerlines", "omni_host_trace_centerlines", "omni_trace_results",
     "omni_kmeans_lab_batch", "omni_color_edge_packed_frames", "omni_host_color_edge_packed_frames",
+    "omni_png_bound", "omni_png_encode", "omni_host_png_encode",
 ]
 
 
@@ -105,6 +109,9 @@ def lib():
         "omni_trace_centerlines": ([vp, u8p, i, i, i, sz, sz, i64p, vp], i),
         "omni_host_trace_centerlines": ([vp, u8p, i, i, i, sz, sz, i64p], i),
         "omni_trace_results": ([vp, vp, vp, vp], i),
+        "omni_png_bound": ([i, i, i], sz),
+        "omni_png_encode": ([vp, u8p, i, sz, i, i, sz, i, u8p, sz, i64p, vp], i),
+        "omni_host_png_encode": ([vp, u8p, i, sz, i, i, sz, i, u8p, sz, i64p], i),
     }
     for name, (args, res) in sig.items():
         fn = getattr(L, name)

@@ -500,6 +500,39 @@ class Engine:
             c0, l0, p0 = c0 + nc, l0 + npath, p0 + npt
         return out
 
+    # ---- PNG files of stages 01-03 (01:30, 02:156, 03:37, 03:60-111) ------------------------------------
+    def png_encode(self, images: torch.Tensor, fmt, w: int | None = None) -> list:
+        """Device images -> one PNG file (bytes) each, encoded on the GPU (omni_png_encode).  fmt capi.PNG_GRAY1 ("gray1"):
+        packed MSB-first rows [H, RB] or [n, H, RB] (w: pixels per row, default 8 * RB); capi.PNG_BGR8 ("bgr8"): [H, W, 3] or
+        [n, H, W, 3] BGR.  Any row / image strides.  Synchronises the current stream."""
+        if not (isinstance(images, torch.Tensor) and images.is_cuda and images.dtype == torch.uint8):
+            raise TypeError("expected a CUDA uint8 tensor")
+        fmt = _png_format(fmt)
+        n, h, w, pitch, stride = _png_geometry(tuple(images.shape), tuple(images.stride()), fmt, w)
+        cap = n * int(self._L.omni_png_bound(h, w, fmt))
+        out = torch.empty(max(1, cap), dtype=torch.uint8, device=images.device)
+        sizes = np.zeros(n, np.int64)
+        capi.check(self._L.omni_png_encode(self._h, images.data_ptr(), n, stride, h, w, pitch, fmt, out.data_ptr(), cap,
+                                           sizes.ctypes.data_as(C.POINTER(C.c_int64)), self._stream()))
+        return _png_split(out[:int(sizes.sum())].cpu().numpy(), sizes)
+
+    def host_png_encode(self, images: np.ndarray, fmt, w: int | None = None) -> list:
+        """Host-buffer form of png_encode (NumPy in, bytes out; ctypes + NumPy only): one H2D copy of the pixels, one D2H copy
+        of the compressed files."""
+        a = np.asarray(images)
+        if a.dtype != np.uint8:
+            raise TypeError("expected a uint8 array")
+        fmt = _png_format(fmt)
+        if a.ndim == 0 or any(s < 0 for s in a.strides) or a.strides[-1] != 1:
+            a = np.ascontiguousarray(a)
+        n, h, w, pitch, stride = _png_geometry(a.shape, a.strides, fmt, w)
+        cap = n * int(self._L.omni_png_bound(h, w, fmt))
+        out = np.empty(max(1, cap), np.uint8)
+        sizes = np.zeros(n, np.int64)
+        capi.check(self._L.omni_host_png_encode(self._h, a.ctypes.data, n, stride, h, w, pitch, fmt, out.ctypes.data, cap,
+                                                sizes.ctypes.data_as(C.POINTER(C.c_int64))))
+        return _png_split(out, sizes)
+
     def last_hysteresis_passes(self) -> int:
         return int(self._L.omni_last_hysteresis_passes(self._h))
 
@@ -590,6 +623,40 @@ def _as_u8(a: np.ndarray, ch: int) -> np.ndarray:
     if a.strides[2] != 1 or a.strides[1] != ch:
         a = np.ascontiguousarray(a)
     return a
+
+
+def _png_format(fmt) -> int:
+    names = {"gray1": capi.PNG_GRAY1, "bgr8": capi.PNG_BGR8}
+    if isinstance(fmt, str):
+        if fmt.lower() not in names:
+            raise ValueError(f"unknown PNG format {fmt!r} (gray1, bgr8)")
+        return names[fmt.lower()]
+    return int(fmt)             # other values reach the C call, which reports them
+
+
+def _png_geometry(shape, strides, fmt: int, w):
+    """(n, h, w, row pitch, image stride) of one image or a stack of images for omni_png_encode (strides in bytes)."""
+    batched = len(shape) == (3 if fmt == capi.PNG_GRAY1 else 4)
+    if fmt == capi.PNG_BGR8:
+        if len(shape) not in (3, 4) or shape[-1] != 3 or strides[-1] != 1 or strides[-2] != 3:
+            raise ValueError("PNG_BGR8 expects [H, W, 3] or [n, H, W, 3] uint8 with packed pixels")
+        if w is not None and int(w) != shape[-2]:
+            raise ValueError(f"w={w} does not match the image width {shape[-2]}")
+        h, w, pitch = shape[-3], shape[-2], strides[-3]
+    else:
+        if len(shape) not in (2, 3) or strides[-1] != 1:
+            raise ValueError("PNG_GRAY1 expects packed rows [H, RB] or [n, H, RB] uint8 with unit column stride")
+        h, rb, pitch = shape[-2], shape[-1], strides[-2]
+        w = 8 * rb if w is None else int(w)
+        if (w + 7) // 8 > rb:
+            raise ValueError(f"w={w} needs {(w + 7) // 8} bytes per row, the rows have {rb}")
+    n = shape[0] if batched else 1
+    return n, h, w, pitch, (strides[0] if batched else 0)
+
+
+def _png_split(buf: np.ndarray, sizes: np.ndarray) -> list:
+    ends = np.cumsum(sizes)
+    return [buf[e - s:e].tobytes() for s, e in zip(sizes.tolist(), ends.tolist())]
 
 
 def pinned_empty(shape, dtype=np.uint8) -> np.ndarray:

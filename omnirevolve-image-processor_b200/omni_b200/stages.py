@@ -10,9 +10,11 @@ and error behaviour), with the per-pixel arithmetic done by libomni_b200's CUDA 
     03_edge_detect.save_edges_composite(cfg)    save_edges_composite(cfg)
     process_colors.assign_labels(img, pal)      assign_labels(img, pal)
 
-Image decode/encode (cv2.imread / cv2.imwrite) and cv2.kmeans stay host-side library calls exactly as in
-the reference: PNG files and k-means centres are the stage boundary / inputs, not the data-parallel path.
-There is no CPU fallback for the pixel work: without a GPU every function here raises.
+Image decode (cv2.imread) and cv2.kmeans stay host-side library calls exactly as in the reference: PNG files and k-means
+centres are the stage boundary / inputs, not the data-parallel path.  The PNG files these stages write are encoded on the GPU
+(omni_host_png_encode): the K layer files of a stage in one call, resized.png and edges_composite.png in one call each;
+OMNI_B200_PNG_BITS=8 keeps the cv2.imwrite files of before.  There is no CPU fallback for the pixel work: without a GPU every
+function here raises.
 """
 from __future__ import annotations
 
@@ -55,7 +57,7 @@ def resize_main(cfg) -> str:
     cfg.ensure_output_dirs()
     out = resize_if_needed(cfg.input_image, cfg)
     path = os.path.join(cfg.output_dir, "resized.png")
-    cv2.imwrite(path, out)
+    _write_bgr_png(path, out, _encode_resized)
     print(f"Saved: {path}")
     return path
 
@@ -187,18 +189,65 @@ def _lab_to_bgr(lab3) -> tuple:
     return int(bgr[0]), int(bgr[1]), int(bgr[2])
 
 
-def _write_layer_png(path: str, plane_u8=None, bits=None, w=None) -> None:
-    """mask.png / edges.png: a 1-bit greyscale PNG (decodes through cv2.imread to the same {0,255} pixels; see omni_b200/png1.py)
-    unless OMNI_B200_PNG_BITS=8.  Give either the u8 plane or its MSB-first packed rows."""
+# ---- PNG files ------------------------------------------------------------------------------------------------------------
+# The encoders of the files, one function per kind of file (tools/png_probe.py swaps in the host encoders of before to compare).
+def _encode_layers(bits: np.ndarray, w: int) -> list:
+    """mask.png / edges.png of all K layers of a stage: packed MSB-first rows [K, H, ceil(w/8)] -> K 1-bit greyscale PNG files,
+    in ONE GPU call (calls on one engine must not overlap, so never from the I/O threads)."""
+    return get_engine().host_png_encode(bits, "gray1", w)
+
+
+def _encode_resized(img: np.ndarray) -> bytes:
+    """resized.png (01:30)."""
+    return get_engine().host_png_encode(img, "bgr8")[0]
+
+
+def _encode_composite(canvas: np.ndarray) -> bytes:
+    """edges_composite.png (03:60-111)."""
+    return get_engine().host_png_encode(canvas, "bgr8")[0]
+
+
+def _write_bytes(path: str, data: bytes) -> None:
+    with open(path, "wb") as fh:
+        fh.write(data)
+
+
+def _write_bgr_png(path: str, img: np.ndarray, encode, cv2_params=()) -> None:
+    """A BGR file: encoded on the GPU, or by cv2.imwrite with `cv2_params` as before under OMNI_B200_PNG_BITS=8."""
     from . import png1
     if png1.use_1bit():
-        if bits is None:
-            bits, w = np.packbits(plane_u8 > 0, axis=1), plane_u8.shape[1]
-        png1.write_png1(path, bits, w)
+        _write_bytes(path, encode(img))
     else:
-        if plane_u8 is None:
-            plane_u8 = png1.unpack_rows(bits, w)
-        cv2.imwrite(path, plane_u8)
+        cv2.imwrite(path, img, list(cv2_params))
+
+
+def _write_layer_pngs(cfg, paths, planes=None, bits=None, w=None) -> None:
+    """mask.png / edges.png files of a stage: 1-bit greyscale PNGs (decode through cv2.imread to the same {0,255} pixels; see
+    omni_b200/png1.py) encoded in one call from this thread, written by the I/O pool; unless OMNI_B200_PNG_BITS=8, which keeps the
+    8-bit cv2.imwrite files.  Give the u8 planes [K, H, W] (or a list of planes of any sizes) or their MSB-first packed rows."""
+    from . import png1
+    paths = list(paths)
+    if not paths:
+        return
+    if png1.use_1bit():
+        if bits is not None:
+            files = _encode_layers(bits, w)
+        elif isinstance(planes, np.ndarray) and planes.ndim == 3:
+            files = _encode_layers(np.packbits(planes > 0, axis=-1), planes.shape[-1])
+        else:                                           # planes of different sizes: one call per size
+            files = [_encode_layers(np.packbits(p > 0, axis=-1)[None], p.shape[-1])[0] for p in planes]
+        work = list(zip(paths, files))
+        fn = lambda pf: _write_bytes(*pf)               # noqa: E731
+    else:
+        if planes is None:
+            planes = [png1.unpack_rows(b, w) for b in bits]
+        work = list(zip(paths, planes))
+        fn = lambda pp: cv2.imwrite(*pp)                # noqa: E731
+    if len(work) == 1:
+        fn(work[0])
+        return
+    with _io_pool(cfg, len(work)) as pool:              # the file writes (and the 8-bit encodes) in parallel
+        list(pool.map(fn, work))
 
 
 def _swatch_extract(cfg, img, names) -> None:
@@ -210,9 +259,10 @@ def _swatch_extract(cfg, img, names) -> None:
     import torch
     cols = [[int(v) for v in colors[i]] for i in range(len(names))]
     masks = get_engine().swatch_masks(torch.from_numpy(np.ascontiguousarray(img)).cuda(), cols, tol).cpu().numpy()
-    for i, name in enumerate(names):
+    for name in names:
         os.makedirs(os.path.join(cfg.output_dir, name), exist_ok=True)
-        _write_layer_png(os.path.join(cfg.output_dir, name, "mask.png"), plane_u8=masks[i])
+    _write_layer_pngs(cfg, [os.path.join(cfg.output_dir, name, "mask.png") for name in names], planes=masks[:len(names)])
+    for i, name in enumerate(names):
         print(f"Extracted (swatch): {name} | nz={int(np.count_nonzero(masks[i]))}")
     print("Color extraction: done.")
 
@@ -271,10 +321,9 @@ def color_extract_main(cfg, img=None) -> dict:
     palette = {}
     for name, _k in mapping:
         os.makedirs(os.path.join(cfg.output_dir, name), exist_ok=True)
-    with _io_pool(cfg, len(mapping)) as pool:                      # K PNG encodes in parallel (zlib / cv2 release the GIL)
-        list(pool.map(lambda nk: _write_layer_png(os.path.join(cfg.output_dir, nk[0], "mask.png"),
-                                                  plane_u8=None if planes is None else planes[nk[1]],
-                                                  bits=None if bits is None else bits[nk[1]], w=w), mapping))
+    paths = [os.path.join(cfg.output_dir, nk[0], "mask.png") for nk in mapping]
+    ks = [k for _n, k in mapping]
+    _write_layer_pngs(cfg, paths, planes=None if planes is None else planes[ks], bits=None if bits is None else bits[ks], w=w)
     for name, k in mapping:
         lab = centers_sorted[k]
         palette[name] = {
@@ -319,8 +368,7 @@ def _handoff_drop(cfg) -> None:
 def _handoff_write(cfg, ec, mapping, edge_bits, counts, w) -> None:
     names = list(cfg.color_names)
     plane_of = dict(mapping)
-    with _io_pool(cfg, len(names)) as pool:
-        list(pool.map(lambda n: _write_layer_png(os.path.join(cfg.output_dir, n, _HIDDEN_EDGES), bits=edge_bits[plane_of[n]], w=w), names))
+    _write_layer_pngs(cfg, [os.path.join(cfg.output_dir, n, _HIDDEN_EDGES) for n in names], bits=edge_bits[[plane_of[n] for n in names]], w=w)
     note = {"edge": _edge_keys(cfg), "color_names": names, "colors": [list(map(int, c)) for c in list(cfg.colors)],
             "masks": {n: list(_stamp(os.path.join(cfg.output_dir, n, "mask.png"))) for n in names},
             "edge_nz": {n: int(counts[plane_of[n], 2]) for n in names}, "composite": False}
@@ -328,7 +376,7 @@ def _handoff_write(cfg, ec, mapping, edge_bits, counts, w) -> None:
         from . import png1
         stack = np.stack([png1.unpack_rows(edge_bits[plane_of[n]], w) for n in names])
         canvas = get_engine().host_edges_composite(stack, [tuple(cfg.colors[i]) for i in range(len(names))])
-        cv2.imwrite(os.path.join(cfg.output_dir, _HIDDEN_COMPOSITE), canvas, [cv2.IMWRITE_PNG_COMPRESSION, 1])
+        _write_bgr_png(os.path.join(cfg.output_dir, _HIDDEN_COMPOSITE), canvas, _encode_composite, [cv2.IMWRITE_PNG_COMPRESSION, 1])
         note["composite"] = True
     with open(os.path.join(cfg.output_dir, _HANDOFF), "w", encoding="utf-8") as fh:
         json.dump(note, fh)
@@ -383,13 +431,18 @@ def edge_detect_main(cfg) -> None:
 def front_half_main(cfg) -> None:
     """Stages 01 -> 02 -> 03 in ONE process (SURVEY 8f rank 3: in-memory hand-off): the same files and log lines as the three stage
     scripts run one after the other, but one interpreter start and one CUDA context, the resized image goes from stage 01 to
-    stage 02 as an array (resized.png is written in the background, not decoded again), and stage 03 publishes the edge planes the
-    fused stage-02 call has produced.  `python front_half.py` with CONFIG_PATH set, in place of steps 1-3 of pipeline.py."""
+    stage 02 as an array (resized.png is encoded on the GPU and written in the background, not decoded again), and stage 03
+    publishes the edge planes the fused stage-02 call has produced.  `python front_half.py` with CONFIG_PATH set, in place of
+    steps 1-3 of pipeline.py."""
     import threading
+    from . import png1
     cfg.ensure_output_dirs()
     img = resize_if_needed(cfg.input_image, cfg)
     path = os.path.join(cfg.output_dir, "resized.png")
-    writer = threading.Thread(target=cv2.imwrite, args=(path, img))       # cv2 releases the GIL while it encodes
+    if png1.use_1bit():                                 # encoded here (the engine is this thread's), written in the background
+        writer = threading.Thread(target=_write_bytes, args=(path, _encode_resized(img)))
+    else:
+        writer = threading.Thread(target=cv2.imwrite, args=(path, img))   # cv2 releases the GIL while it encodes
     writer.start()
     try:
         color_extract_main(cfg, img=img)
@@ -421,7 +474,7 @@ def process_color(color_name: str, cfg):
     mask = _read_mask(color_name, cfg)
     edges = get_engine().host_edges(mask[None], EdgeConfig.from_cfg(cfg))[0]
     out_path = os.path.join(cfg.output_dir, color_name, "edges.png")
-    _write_layer_png(out_path, plane_u8=edges)
+    _write_layer_pngs(cfg, [out_path], planes=edges[None])
     print(f"Edges extracted: {color_name} | nz={int(np.count_nonzero(edges))}")
     return color_name, out_path
 
@@ -439,8 +492,8 @@ def detect_all_edges(cfg) -> list:
     """03_edge_detect.py:42-48.  The reference fans layers out over a process pool; here all layers of
     equal size go through ONE batched GPU call (layers are the plane dimension of omni_edges)."""
     names = list(cfg.color_names)
-    # PNG decode / encode is what is left of this stage's wall time: spread it over threads the way the reference spreads
-    # layers over cfg.n_cores processes (cv2 releases the GIL); errors surface in layer order like in a serial loop
+    # PNG decode is what is left of this stage's wall time: spread it over threads the way the reference spreads layers over
+    # cfg.n_cores processes (cv2 releases the GIL); errors surface in layer order like in a serial loop
     with _io_pool(cfg, len(names)) as pool:
         masks = list(pool.map(lambda n: _read_mask(n, cfg), names))
     results = []
@@ -450,8 +503,7 @@ def detect_all_edges(cfg) -> list:
     else:                                   # hand-edited masks of different sizes: one call per layer
         edges = [get_engine().host_edges(m[None], EdgeConfig.from_cfg(cfg))[0] for m in masks]
     paths = [os.path.join(cfg.output_dir, n, "edges.png") for n in names]
-    with _io_pool(cfg, len(names)) as pool:
-        list(pool.map(lambda pe: _write_layer_png(pe[0], plane_u8=pe[1]), zip(paths, edges)))
+    _write_layer_pngs(cfg, paths, planes=edges)
     for n, e, out_path in zip(names, edges, paths):
         print(f"Edges extracted: {n} | nz={int(np.count_nonzero(e))}")
         results.append((n, out_path))
@@ -527,7 +579,7 @@ def save_edges_composite(cfg) -> str:
         canvas = get_engine().host_edges_composite(stack, [name_to_bgr[n] for n in order])
     else:
         canvas = np.full((h, w, 3), 255, np.uint8)
-    cv2.imwrite(out_path, canvas, [cv2.IMWRITE_PNG_COMPRESSION, 1])      # same pixels, a third of the encode time
+    _write_bgr_png(out_path, canvas, _encode_composite, [cv2.IMWRITE_PNG_COMPRESSION, 1])
     print(f"Edges composite saved: {out_path}")
     return out_path
 
