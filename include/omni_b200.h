@@ -144,9 +144,10 @@ int omni_swatch_masks(omni_ctx *ctx, const uint8_t *d_bgr, int h, int w, size_t 
  * seeding (3 trials per centre), Lloyd iterations until no centre moves by more than eps or max_iter, best of `attempts` by
  * compactness -- on the 8-bit Lab values of the pixels h_sample_idx[0 .. n_samples) (host array; pass the reference's own
  * `default_rng(42).choice(h*w, 200000, replace=False)`; NULL = every pixel, h*w <= 2^24).  cv2.kmeans draws from OpenCV's global
- * RNG, so its centres cannot be reproduced bit for bit; this call is deterministic for a given seed (integer accumulation) and
- * returns centres whose compactness (sum of squared distances of the samples to their centre, *h_compactness if not NULL) is
- * within 2 % of cv2.kmeans' on the same sample (tests/test_gpu_kmeans.py).  Synchronises the stream (centres go to the host). */
+ * RNG, so its centres cannot be reproduced bit for bit; this call is deterministic for a given seed (integer accumulation): its
+ * centres and compactness (sum of squared distances of the samples to their centre, *h_compactness if not NULL) equal bit for
+ * bit those of oracle/kmeans_model.py, a NumPy restatement of the kernels (tests/test_gpu_kmeans_exact.py), and the compactness
+ * is within 2 % of cv2.kmeans' on the same sample (tests/test_gpu_kmeans.py).  Synchronises the stream (centres go to the host). */
 int omni_kmeans_lab(omni_ctx *ctx, const uint8_t *d_bgr, int h, int w, size_t pitch, const int32_t *h_sample_idx, int n_samples,
                     int K, int attempts, int max_iter, double eps, uint64_t seed, float *h_centers, double *h_compactness, void *stream);
 /* The same for n_frames equally sized frames, frame f at d_bgr + f*frame_stride, each clustered on its own with the same sample

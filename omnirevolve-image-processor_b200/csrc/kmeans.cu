@@ -6,9 +6,10 @@
 // one keeps the structure (same sample -- the caller passes the reference's own indices --, kmeans++ with 3 trials per centre,
 // Lloyd to the same stopping rule, best of `attempts` by compactness) and is DETERMINISTIC: the sample's 8-bit Lab values are
 // accumulated as integers, the compactness in fixed point, so no result depends on the order of the atomics.
-// Contract (tests/test_gpu_kmeans.py): the compactness of the returned centres is within 2 % of cv2.kmeans' on the same sample;
-// labels and masks then follow from the usual exact assignment to THESE centres.  Off by default: the drop-in stage script uses
-// it only when OMNI_B200_KMEANS=gpu.
+// Contract: the centres and the compactness are pinned bit for bit to oracle/kmeans_model.py, a NumPy restatement of these kernels
+// (tests/test_gpu_kmeans_exact.py; exact because of --fmad=false, integer sums and the fixed-point compactness), and their
+// compactness is within 2 % of cv2.kmeans' on the same sample (tests/test_gpu_kmeans.py); labels and masks then follow from the
+// usual exact assignment to THESE centres.  Off by default: the drop-in stage script uses it only when OMNI_B200_KMEANS=gpu.
 //
 // Every (frame, attempt) pair is an independent RUN with its own state and seeding scratch; all runs of a chunk of frames go
 // through the same launches (run index = blockIdx.y of the Lloyd assignment, one CTA per run in the seeding, one thread per run in

@@ -21,6 +21,24 @@ def uniform_img(H, W, seed):
     return np.random.default_rng(seed).integers(0, 256, (H, W, 3), dtype=np.uint8)
 
 
+KMEANS_TOL = 0.02          # k-means quality bound: compactness within 2 % of cv2.kmeans' on the same sample
+
+
+def lab_sample(img, limit=200_000):
+    """02_color_extract.py:35-42: the seeded subsample (None: every pixel) and its 8-bit Lab values from cv2."""
+    n = img.shape[0] * img.shape[1]
+    idx = np.random.default_rng(42).choice(n, size=limit, replace=False) if n > limit else None
+    flat = img.reshape(-1, 3) if idx is None else img.reshape(-1, 3)[idx]
+    lab = cv2.cvtColor(np.ascontiguousarray(flat).reshape(-1, 1, 3), cv2.COLOR_BGR2LAB).reshape(-1, 3).astype(np.float32)
+    return idx, lab
+
+
+def compactness(lab, centers):
+    """Sum over the samples of the squared distance to the nearest centre, in float64."""
+    d = ((lab[:, None, :].astype(np.float64) - centers[None].astype(np.float64)) ** 2).sum(axis=2)
+    return float(d.min(axis=1).sum())
+
+
 def smooth_u8(H, W, seed, k=7):
     g = np.random.default_rng(seed).integers(0, 256, (H + 2 * k, W + 2 * k), dtype=np.uint8)
     return np.ascontiguousarray(cv2.GaussianBlur(g, (k, k), 0)[k:k + H, k:k + W])

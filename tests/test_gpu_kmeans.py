@@ -11,11 +11,10 @@ import cv2
 import numpy as np
 import pytest
 
-from helpers import synth, uniform_img
+from helpers import KMEANS_TOL as TOL, compactness as _compactness, lab_sample as _sample, synth, uniform_img
 
 pytestmark = pytest.mark.gpu
 torch = pytest.importorskip("torch")
-TOL = 0.02
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
@@ -25,20 +24,6 @@ def eng():
     e = omni_b200.Engine(0)
     yield e
     e.close()
-
-
-def _sample(img, limit=200_000):
-    """02_color_extract.py:35-42: the seeded subsample and its 8-bit Lab values."""
-    n = img.shape[0] * img.shape[1]
-    idx = np.random.default_rng(42).choice(n, size=limit, replace=False) if n > limit else None
-    flat = img.reshape(-1, 3) if idx is None else img.reshape(-1, 3)[idx]
-    lab = cv2.cvtColor(np.ascontiguousarray(flat).reshape(-1, 1, 3), cv2.COLOR_BGR2LAB).reshape(-1, 3).astype(np.float32)
-    return idx, lab
-
-
-def _compactness(lab, centers):
-    d = ((lab[:, None, :].astype(np.float64) - centers[None].astype(np.float64)) ** 2).sum(axis=2)
-    return float(d.min(axis=1).sum())
 
 
 @pytest.mark.parametrize("K", [2, 4, 8, 16])
