@@ -292,12 +292,28 @@ int omni_skeleton_degree(omni_ctx *ctx, const uint8_t *d_skel, int K, int h, int
  * same points in the same order.
  * The output size is found on the device, so the call SYNCHRONISES the stream.  h_plane_info (optional, 4*K int64): per plane
  * [total_fg, components, polylines, points].  The results stay in the ctx until the next omni_trace_centerlines /
- * omni_host_trace_centerlines call on it; omni_trace_results copies them out. */
+ * omni_host_trace_centerlines / omni_[host_]centerlines_packed call on it; omni_trace_results copies them out. */
 int omni_trace_centerlines(omni_ctx *ctx, const uint8_t *d_skel, int K, int h, int w, size_t plane_stride, size_t pitch,
                            int64_t *h_plane_info, void *stream);
 /* Host-buffer form: h_skel is copied in, then as omni_trace_centerlines. */
 int omni_host_trace_centerlines(omni_ctx *ctx, const uint8_t *h_skel, int K, int h, int w, size_t plane_stride, size_t pitch,
                                 int64_t *h_plane_info);
+/* Packed edge planes -> centrelines, any number of planes: plane p (layer p % K of frame p / K for a batch of frames) at
+ * d_edge_bits + p*plane_stride, rows pitch bytes apart (>= ceil(w / 8); plane_stride >= pitch * h), bit_order as for
+ * omni_color_edge_packed -- what omni_color_edge_packed / omni_host_color_edge_packed write.  Each plane's result equals
+ * omni_thin_zhangsuen_packed(max_iter) on it, unpacked to {0,255} bytes, then omni_trace_centerlines on it: the same points,
+ * polylines, component rows and h_plane_info row.  The planes go through in chunks -- at least 32 planes, more while the labels of a
+ * chunk (8 bytes per 2x2 block and plane) fit 256 MiB -- each thinned (OMNI_MAX_K planes per launch), unpacked and traced with all
+ * its components in one set of walk launches; so small frames fill the GPU that one frame's components leave idle.  The input is
+ * not modified.  h_plane_info (optional, 4*n_planes int64) and the results as for omni_trace_centerlines: omni_trace_results copies
+ * them out, planes in order.  Synchronises the stream.  Scratch: workspace slots 3 (host form), 7-10 and 12 of the ctx, grown on
+ * demand and kept (slot 10, the polylines, grows with the output); omni_workspace_bytes / omni_ctx_reserve do not cover them. */
+int omni_centerlines_packed(omni_ctx *ctx, const uint8_t *d_edge_bits, int n_planes, int h, int w, size_t plane_stride, size_t pitch,
+                            int bit_order, int max_iter, int64_t *h_plane_info, void *stream);
+/* Host-buffer form: each chunk's planes are copied in (on the ctx's own stream), then as omni_centerlines_packed; returns when the
+ * results are in the ctx. */
+int omni_host_centerlines_packed(omni_ctx *ctx, const uint8_t *h_edge_bits, int n_planes, int h, int w, size_t plane_stride,
+                                 size_t pitch, int bit_order, int max_iter, int64_t *h_plane_info);
 /* Copies the result of the last trace into caller buffers (host or device memory; any may be NULL) and returns when they hold it:
  * h_points: int32 [points][2] = (x, y) of every polyline, planes in order, components in label order (cv2's), polylines in the
  * reference's order; h_path_len: int32 [polylines], the number of points of each; h_comp: int32 [components][6] = cv2's stats row

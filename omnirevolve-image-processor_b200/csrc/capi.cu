@@ -1119,6 +1119,37 @@ extern "C" int omni_host_trace_centerlines(omni_ctx *ctx, const uint8_t *h_skel,
     return omni_trace_centerlines(ctx, d, K, h, w, dplane, dp, h_plane_info, ctx->stream);
 }
 
+// ---- packed edge planes -> thinning -> centrelines, any number of planes (trace.cu) -------------------------------------------
+static int centerlines_args(const char *who, const void *bits, int n_planes, int h, int w, size_t plane_stride, size_t pitch,
+                            int bit_order, int max_iter)
+{
+    OMNI_REQUIRE(bits && n_planes >= 1 && h > 0 && w > 0, "%s: bad arguments", who);
+    OMNI_REQUIRE(pitch >= (size_t)(w + 7) / 8 && plane_stride >= pitch * h, "%s: pitch smaller than a row or plane stride smaller than a plane", who);
+    OMNI_REQUIRE(bit_order == OMNI_BITS_LSB_FIRST || bit_order == OMNI_BITS_MSB_FIRST, "%s: bad bit order", who);
+    OMNI_REQUIRE(max_iter >= 0 && max_iter <= 100000, "%s: max_iter %d out of range", who, max_iter);
+    OMNI_REQUIRE((long long)((w + 1) / 2) * ((h + 1) / 2) * centerlines_chunk(h, w, n_planes) < INT32_MAX,
+                 "%s: planes of %d x %d are too large", who, w, h);
+    return OMNI_OK;
+}
+
+extern "C" int omni_centerlines_packed(omni_ctx *ctx, const uint8_t *d_edge_bits, int n_planes, int h, int w, size_t plane_stride,
+                                       size_t pitch, int bit_order, int max_iter, int64_t *h_plane_info, void *stream)
+{
+    OMNI_TRY(set_device(ctx));
+    OMNI_TRY(centerlines_args("omni_centerlines_packed", d_edge_bits, n_planes, h, w, plane_stride, pitch, bit_order, max_iter));
+    return centerlines_packed_run(ctx, d_edge_bits, nullptr, n_planes, h, w, plane_stride, pitch, bit_order, max_iter, h_plane_info,
+                                  (cudaStream_t)stream);
+}
+
+extern "C" int omni_host_centerlines_packed(omni_ctx *ctx, const uint8_t *h_edge_bits, int n_planes, int h, int w, size_t plane_stride,
+                                            size_t pitch, int bit_order, int max_iter, int64_t *h_plane_info)
+{
+    OMNI_TRY(set_device(ctx));
+    OMNI_TRY(centerlines_args("omni_host_centerlines_packed", h_edge_bits, n_planes, h, w, plane_stride, pitch, bit_order, max_iter));
+    return centerlines_packed_run(ctx, nullptr, h_edge_bits, n_planes, h, w, plane_stride, pitch, bit_order, max_iter, h_plane_info,
+                                  ctx->stream);
+}
+
 extern "C" int omni_trace_results(omni_ctx *ctx, int32_t *h_points, int32_t *h_path_len, int32_t *h_comp)
 {
     OMNI_TRY(set_device(ctx));

@@ -56,12 +56,12 @@ struct ResizeTab {
     ResizeTabDev dev{};
 };
 
-#define OMNI_WS_SLOTS 12
+#define OMNI_WS_SLOTS 13
 struct omni_ctx {
     int device = 0;
     int fast = 1;
     // grow-only device scratch
-    void *ws[OMNI_WS_SLOTS] = {};          // 0-2 generic planes, 3 host staging, 4 bit-planes, 5 misc, 6 edge run lists, 7-10 trace.cu, 11 png_encode.cu
+    void *ws[OMNI_WS_SLOTS] = {};          // 0-2 generic planes, 3 host staging, 4 bit-planes, 5 misc, 6 edge run lists, 7-10 trace.cu, 11 png_encode.cu, 12 thinned / byte planes of omni_centerlines_packed
     size_t ws_bytes[OMNI_WS_SLOTS] = {};
     int *d_flags = nullptr;          // 64 ints of device flags / counters
     unsigned long long *d_counts = nullptr;   // 4*OMNI_MAX_K counters
@@ -120,9 +120,11 @@ struct omni_ctx {
     size_t pk_counts_cap = 0;                  // groups of 3 * OMNI_MAX_K counts
     int pipeline = 1;                          // fused colour+edge call: 1 = sparse generation (label_pipe.cu), 0 = dense generation
     u8 *d_rgb_boxes = nullptr;                 // exact Lab box of every 4x4x4 RGB cell (centre-independent, built on first use)             // co-resident CTAs of the cooperative hysteresis kernel (0 = not queried yet)
-    // result of the last omni_trace_centerlines call: polylines in ws[10], sizes and per-component rows on the host
+    // result of the last omni_trace_centerlines / omni_centerlines_packed call: polylines in ws[10] (points from offset 0, path
+    // lengths from trace_lens_off), sizes and per-component rows on the host
     int trace_valid = 0, trace_K = 0;
     long long trace_points = 0, trace_paths = 0;
+    size_t trace_lens_off = 0;
     std::vector<long long> trace_info;         // per plane: total_fg, components, polylines, points
     std::vector<int32_t> trace_comp;           // per component: left, top, width, height, area, polylines
 };
@@ -141,6 +143,11 @@ int omni_ws_reserve(omni_ctx *ctx, int slot, size_t bytes);
 int trace_run(omni_ctx *ctx, const u8 *d_skel, int K, int h, int w, size_t plane_stride, size_t pitch, int64_t *h_info,
               cudaStream_t st);
 int trace_results(omni_ctx *ctx, int32_t *points, int32_t *path_len, int32_t *comp);
+// omni_centerlines_packed: planes per chunk (at least 32, more while the labels of a chunk fit 256 MiB), and the run (capi.cu
+// checks the arguments; h_bits != NULL: host planes, each chunk copied in first; synchronises st)
+int centerlines_chunk(int h, int w, int n_planes);
+int centerlines_packed_run(omni_ctx *ctx, const u8 *d_bits, const u8 *h_bits, int n_planes, int h, int w, size_t plane_stride,
+                           size_t pitch, int bit_order, int max_iter, int64_t *h_info, cudaStream_t st);
 // PNG encoder (png_encode.cu): a segment holds at most PNG_SEG_MAX filtered bytes (one stored block) and PNG_SEG_ROWS rows
 constexpr int PNG_SEG_MAX = 61440;
 constexpr int PNG_SEG_ROWS = 256;

@@ -32,6 +32,7 @@ EXPORTS = [
     "omni_trace_centerlines", "omni_host_trace_centerlines", "omni_trace_results",
     "omni_kmeans_lab_batch", "omni_color_edge_packed_frames", "omni_host_color_edge_packed_frames",
     "omni_png_bound", "omni_png_encode", "omni_host_png_encode",
+    "omni_centerlines_packed", "omni_host_centerlines_packed",
 ]
 
 
@@ -109,6 +110,8 @@ def lib():
         "omni_trace_centerlines": ([vp, u8p, i, i, i, sz, sz, i64p, vp], i),
         "omni_host_trace_centerlines": ([vp, u8p, i, i, i, sz, sz, i64p], i),
         "omni_trace_results": ([vp, vp, vp, vp], i),
+        "omni_centerlines_packed": ([vp, u8p, i, i, i, sz, sz, i, i, i64p, vp], i),
+        "omni_host_centerlines_packed": ([vp, u8p, i, i, i, sz, sz, i, i, i64p], i),
         "omni_png_bound": ([i, i, i], sz),
         "omni_png_encode": ([vp, u8p, i, sz, i, i, sz, i, u8p, sz, i64p, vp], i),
         "omni_host_png_encode": ([vp, u8p, i, sz, i, i, sz, i, u8p, sz, i64p], i),

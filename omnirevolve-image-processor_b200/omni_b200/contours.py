@@ -11,6 +11,8 @@ stats) and walks every component in its own CTA, step for step as the reference 
     trace_centerlines(skel_0_255, layer)      same signature, same polylines in the same order, same progress lines
                                                (04:101-205) except the time-driven "visited n/m px" lines; one GPU call
     trace_layers(skels, names)                 all K layers in one GPU call, each layer's log lines in turn
+    trace_frames(edge_bits, w, K)              packed edge planes of n frames -> thinning + polylines of every layer of every
+                                               frame in one GPU call (omni_centerlines_packed); no log lines
     trace_centerlines(skel, layer, maps=...)   the host walk (a Python restatement of 04:126-200 that takes the degree /
                                                endpoint / junction maps of the whole skeleton and confines every component to
                                                its bounding box): the reference the GPU tracer is tested against
@@ -108,6 +110,17 @@ def trace_centerlines(skel_0_255: np.ndarray, layer: str, maps=None):
     if maps is None:
         return trace_layers(np.asarray(skel_0_255)[None], [layer])[0]
     return _trace_host(skel_0_255, layer, maps)
+
+
+def trace_frames(edge_bits: np.ndarray, w: int, K: int, max_iter: int = MAX_ITER):
+    """Packed edge planes [n*K, H, ceil(w/8)] (MSB-first, as host_color_edge_packed / batch.process_shard_packed return them) ->
+    n lists of K polyline lists: frame f, layer k = trace_centerlines(thinning_zhangsuen(plane f*K + k)), int32 (n,1,2) arrays.
+    All planes go through one GPU call; a batch API, so it prints nothing."""
+    a = np.asarray(edge_bits)
+    if a.ndim != 3 or K < 1 or a.shape[0] % K:
+        raise ValueError(f"expected packed edge planes [n*K, H, RB] with K={K} layers per frame, got {list(a.shape)}")
+    res = get_engine().host_centerlines_packed(a, w, max_iter)
+    return [[r.paths for r in res[f * K:(f + 1) * K]] for f in range(a.shape[0] // K)]
 
 
 def _trace_host(skel_0_255: np.ndarray, layer: str, maps):

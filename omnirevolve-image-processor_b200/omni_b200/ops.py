@@ -485,6 +485,40 @@ class Engine:
                                                        info.ctypes.data_as(C.POINTER(C.c_int64))))
         return self._trace_results(info)
 
+    # ---- stage 04 from packed edge planes: thinning + trace_centerlines, any number of planes --------------------------------
+    def centerlines_packed(self, bits: torch.Tensor, w: int, max_iter: int = 120, msb_first: bool = True) -> list["TraceResult"]:
+        """Packed edge planes [P, H, RB] (CUDA uint8, one bit per pixel, e.g. the edge planes of color_edge_packed for a batch of
+        frames: plane p = layer p % K of frame p // K) -> per plane the TraceResult of trace_centerlines(thin_zhangsuen(plane)).
+        All planes in one call (omni_centerlines_packed).  Synchronises the current stream."""
+        _check_planes(bits)
+        P, h, rb = bits.shape
+        if rb < (w + 7) // 8:
+            raise ValueError("rows too short for w pixels")
+        info = np.zeros((P, 4), np.int64)
+        capi.check(self._L.omni_centerlines_packed(
+            self._h, bits.data_ptr(), P, h, w, bits.stride(0), bits.stride(1), capi.BITS_MSB_FIRST if msb_first else capi.BITS_LSB_FIRST,
+            int(max_iter), info.ctypes.data_as(C.POINTER(C.c_int64)), self._stream()))
+        return self._trace_results(info)
+
+    def host_centerlines_packed(self, bits: np.ndarray, w: int, max_iter: int = 120, msb_first: bool = True) -> list["TraceResult"]:
+        """Host-buffer form of centerlines_packed: NumPy uint8 [P, H, RB] or one [H, RB] (ctypes + NumPy only), e.g. the edge_bits
+        of host_color_edge_packed."""
+        a = np.asarray(bits)
+        if a.ndim == 2:
+            a = a[None]
+        if a.ndim != 3 or a.dtype != np.uint8:
+            raise ValueError("expected uint8 packed planes [P, H, RB] or one [H, RB]")
+        P, h, rb = a.shape
+        if rb < (w + 7) // 8:
+            raise ValueError("rows too short for w pixels")
+        if a.strides[2] != 1 or a.strides[1] < rb or a.strides[0] < a.strides[1] * h:
+            a = np.ascontiguousarray(a)
+        info = np.zeros((P, 4), np.int64)
+        capi.check(self._L.omni_host_centerlines_packed(
+            self._h, a.ctypes.data, P, h, w, a.strides[0], a.strides[1], capi.BITS_MSB_FIRST if msb_first else capi.BITS_LSB_FIRST,
+            int(max_iter), info.ctypes.data_as(C.POINTER(C.c_int64))))
+        return self._trace_results(info)
+
     def _trace_results(self, info: np.ndarray) -> list["TraceResult"]:
         n_comp, n_paths, n_pts = (int(v) for v in info[:, 1:].sum(axis=0))
         pts = np.empty((n_pts, 2), np.int32)
